@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo, one rank per GPU
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write what the last timed step returned
 
 Headline workload (BASELINE.json configs[1]): TIMIT-shaped synthetic utterances (2-4 s, ~40 chars),
 Whisper-medium dimensions with seeded random-init weights, char units, aggr=topk k=10, medfilt_width=3,
@@ -112,7 +113,14 @@ def parse():
     ap.add_argument("--probe-batch", type=int, default=32, help="utterances per probe-sweep step per GPU")
     ap.add_argument("--probe-heads", type=int, default=384, help="heads aligned individually per utterance")
     ap.add_argument("--probe-steps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step of the headline workload returned "
+                         "as DIR/<name>.npy (rank 0, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.aggr is None:
         args.aggr = "mean" if args.workload == "ami" else "topk"
     if args.workload != "timit" or args.model != "medium":
@@ -323,6 +331,37 @@ def pair_roofline(kernel_ms, step_batches, L, H, d, peak):
             "basis": "8*L*H*T*F + 4*L*(T+F)*d per utterance (SURVEY.md 8(d): maps written once and read once for scoring)"}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, results):
+    """Writes what one step of force_align_batch returned, so that two builds can be compared output for output:
+    per utterance the word start / end times, the DTW cost matrix and, for aggr=topk, the kept heads (layer, head)
+    with their scores, each concatenated over the batch in utterance order.  Utterances that came back as the
+    reference's empty sentinel add nothing.  When the matrices would take the dump past DUMP_BYTES, a fixed, seeded
+    sample of their elements is written instead (`matrix_sample`, with the flat positions in `matrix_sample_index`)."""
+    aligned = [r for r in results if not isinstance(r, list)]
+
+    def cat(parts, dtype):
+        return np.concatenate([np.asarray(p, dtype=dtype).ravel() for p in parts]) if parts else np.zeros(0, dtype)
+
+    out = {"start_times": cat([r[1] for r in aligned], np.float64),
+           "end_times": cat([r[2] for r in aligned], np.float64)}
+    if aligned and aligned[0][4] is not None:
+        out["head_scores"] = cat([[s for s, _, _ in r[4]] for r in aligned], np.float32)
+        out["head_layer_head"] = cat([[lh for _, lh, _ in r[4]] for r in aligned], np.float64).reshape(-1, 2)
+    matrix = cat([r[3].numpy() for r in aligned], np.float32)
+    room = DUMP_BYTES - sum(a.nbytes for a in out.values()) - 4096  # 4 KB for the .npy headers
+    if matrix.nbytes <= room:
+        out["matrix"] = matrix
+    else:  # a float32 value and its float64 position per sampled element
+        idx = np.sort(np.random.default_rng(0).choice(matrix.size, room // 12, replace=False))
+        out["matrix_sample"], out["matrix_sample_index"] = matrix[idx], idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     args = parse()
     if args.impl == "reference":
@@ -360,12 +399,8 @@ def main():
     L, H, d = dims.n_text_layer, dims.n_text_head, dims.n_text_state
     unit = "subword" if args.workload == "ami" else "char"
     sot = len(tk.sot_sequence)
-    peaks_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
-    peaks = json.load(open(peaks_path)) if os.path.exists(peaks_path) else {}
-    if "hbm_gbs" in peaks:
-        peak, peak_src = float(peaks["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
-    else:
-        peak, peak_src = 6650.0, "fallback (B200_PROFILING.md)"
+    # one committed figure, so that the roofline fractions of runs on different boxes compare
+    peak, peak_src = 6548.5, "HBM copy bandwidth measured on a B200 (BASELINE.md section 2)"
 
     def barrier():
         if world > 1:
@@ -546,6 +581,8 @@ def main():
             "utterances_aligned": len(local_alignments),
             "configs": extra,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last)
         emit(line)
     if world > 1:
         dist.destroy_process_group()

@@ -166,7 +166,8 @@ WCA_API int wca_head_scores_from_partials(const float *d_partials, const wca_utt
                                   float w_colnorm, float w_rownorm, float *d_scores, wca_stream_t stream);
 
 /* (3b) Top-k head selection.  Replaces timing.py:36 `sorted(scores)[-topk:]`: ascending
- * by (score, layer, head); the last min(topk, n_heads) survive, still ascending.  Writes
+ * by (score, layer, head); the last min(topk, n_heads) survive, still ascending.  -0.0 and +0.0
+ * tie; NaN scores rank below every number, -inf included, and among themselves by index.  Writes
  * head indices (layer*H + head) to d_sel + sel_off and their scores to d_sel_scores +
  * sel_off (n_sel entries per utterance, n_sel taken from the descriptor). */
 WCA_API int wca_topk_heads(const float *d_scores, const wca_utt_t *d_utts, int n_utts, int n_heads, int32_t *d_sel,

@@ -177,6 +177,7 @@ def test_dtw_reproduces_reference_fixture_paths(name, timing, dev):
 @pytest.mark.parametrize("width", [1, 3, 5, 7, 9, 13, 31])
 def test_medfilt_softmax_matches_oracle(width, timing, dev):
     from oracle import ref_path
+    from whisper_char_alignment_b200 import _cabi
 
     g = torch.Generator().manual_seed(width)
     for rows, n_ctx, frames, scale in [(7, 64, 64, 1.0), (40, 1500, 145, 1.0), (33, 1500, 1500, 0.5), (5, 40, 3, 1.0),
@@ -186,6 +187,10 @@ def test_medfilt_softmax_matches_oracle(width, timing, dev):
         got = timing.median_filter_softmax(x.to(dev), frames, width, scale).cpu()
         torch.testing.assert_close(got, want, rtol=2e-6, atol=1e-12)
         torch.testing.assert_close(got.sum(-1), torch.ones(rows), rtol=1e-5, atol=0)
+        # in place (d_out == d_in, ld_in == n_frames): the same bits
+        buf = x[:, :frames].contiguous().to(dev)
+        _cabi.medfilt_softmax(buf, rows, frames, frames, width, scale, buf)
+        assert torch.equal(buf.cpu().view(torch.int32), got.view(torch.int32))
 
 
 def test_medfilt_recovers_the_median_through_log_softmax(timing, dev):

@@ -105,7 +105,7 @@ __global__ void __launch_bounds__(256) head_scores_kernel(const float *__restric
                     s1 += ps[(w * kCols + k) * kWarp + l];
                 }
                 col_part_sum += sqrtf(ss);
-                cov_part += fmaxf(s1, 0.5f);
+                cov_part += s1 < 0.5f ? 0.5f : s1;  // a NaN column sum stays NaN, as in torch.maximum (fmaxf drops it)
             }
             if (ch + 1 < n_chunks) __syncthreads();  // the partials are overwritten by the next chunk
         }
@@ -161,29 +161,36 @@ __global__ void __launch_bounds__(128) scores_from_partials_kernel(const float *
     }
 }
 
-// grid (n_utts), block 256, dynamic smem n_heads floats.  Rank by counting with the
+// Ranking key of a score: an integer ordered like the float, with -0.0 == +0.0 and every NaN (any sign or payload)
+// strictly below -inf.
+__device__ __forceinline__ int32_t topk_key(float v) {
+    if (v != v) return INT32_MIN;
+    const int32_t b = __float_as_int(v == 0.f ? 0.f : v);
+    return b >= 0 ? b : b ^ 0x7fffffff;  // negatives: larger magnitude, smaller key; -inf gives INT32_MIN + 2^23 - 1 > NaN's
+}
+
+// grid (n_utts), block 256, dynamic smem n_heads keys.  Rank by counting with the
 // reference's tuple order (score, layer, head): ties go to the smaller head index.  The order must be TOTAL so that
 // every output slot is written exactly once: a NaN score (non-finite logits upstream) compares false both ways and
 // would give several heads the same rank, leaving `sel` slots uninitialised for aggregate_heads_kernel to
-// dereference.  NaN ranks below every number (the reference's sorted() leaves NaN order unspecified).
+// dereference.  NaN ranks below every number, -inf included, and NaNs among themselves by head index (the reference's
+// sorted() leaves NaN order unspecified).
 __global__ void __launch_bounds__(256) topk_heads_kernel(const float *__restrict__ scores,
                                                          const wca_utt_t *__restrict__ utts, int n_heads,
                                                          int32_t *__restrict__ sel, float *__restrict__ sel_scores) {
-    extern __shared__ float s_sc[];
+    extern __shared__ int32_t s_key[];
     const wca_utt_t u = utts[blockIdx.x];
-    for (int i = threadIdx.x; i < n_heads; i += blockDim.x) {
-        const float v = scores[u.score_off + i];
-        s_sc[i] = (v != v) ? -INFINITY : v;  // ranking key; the reported score stays the original value
-    }
+    for (int i = threadIdx.x; i < n_heads; i += blockDim.x)
+        s_key[i] = topk_key(scores[u.score_off + i]);  // the reported score stays the original value
     __syncthreads();
     const int n_sel = u.n_sel < n_heads ? u.n_sel : n_heads;
     const int first = n_heads - n_sel;
     for (int i = threadIdx.x; i < n_heads; i += blockDim.x) {
-        const float si = s_sc[i];
+        const int32_t ki = s_key[i];
         int rank = 0;
         for (int j = 0; j < n_heads; ++j) {
-            const float sj = s_sc[j];
-            rank += (sj < si) || (sj == si && j < i);
+            const int32_t kj = s_key[j];
+            rank += (kj < ki) || (kj == ki && j < i);
         }
         if (rank >= first) {
             sel[u.sel_off + rank - first] = i;
@@ -289,8 +296,8 @@ int launch_scores_from_partials(const float *d_partials, const wca_utt_t *d_utts
 
 int launch_topk_heads(const float *d_scores, const wca_utt_t *d_utts, int n_utts, int n_heads, int32_t *d_sel,
                       float *d_sel_scores, cudaStream_t stream) {
-    topk_heads_kernel<<<n_utts, 256, n_heads * sizeof(float), stream>>>(d_scores, d_utts, n_heads, d_sel,
-                                                                         d_sel_scores);
+    topk_heads_kernel<<<n_utts, 256, n_heads * sizeof(int32_t), stream>>>(d_scores, d_utts, n_heads, d_sel,
+                                                                           d_sel_scores);
     WCA_LAUNCH_CHECK("topk_heads_kernel");
     return WCA_OK;
 }

@@ -528,8 +528,9 @@ def test_model_forward_is_the_same_with_either_encoder_attention(oracle_models, 
 
 # ------------------------------------------------------------------------ BASELINE.json full-size shapes
 def _planted_qk(rng_seed, n_layers, width, t_list, n_ctx, dev, gain=3.0):
-    """Q / K with a planted monotone structure (token t attends around frame t * F / T) so that the
-    maps are peaky, as real cross-attention is."""
+    """Q / K of plain normal entries, Q scaled by `gain` (logits of std ~gain): fairly peaky maps, but no planted
+    structure and logits far from the lazy-reference rescale of the capture epilogue (tests/test_gpu_capture.py
+    constructs those)."""
     g = torch.Generator(device=dev).manual_seed(rng_seed)
     B, t_max = len(t_list), max(t_list)
     q = [torch.randn(B, t_max, width, device=dev, generator=g) * gain for _ in range(n_layers)]

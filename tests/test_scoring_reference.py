@@ -1,9 +1,10 @@
-"""CPU suite: the float64 references of tests/test_gpu_scoring.py against the fp32 CPU restatement of the reference
-(oracle/ref_path.py), so that the GPU scoring tests rest on references that are themselves checked."""
+"""CPU suite: the float64 references of tests/test_gpu_scoring.py and tests/test_gpu_capture.py against the fp32 CPU
+restatement of the reference (oracle/ref_path.py), so that the GPU tests rest on references that are themselves checked."""
 import numpy as np
 import pytest
 import torch
 
+from test_gpu_capture import ref_capture, ref_logits
 from test_gpu_scoring import NAN, ref_aggregate, ref_head_terms, ref_scores, ref_topk
 
 RTOL = 1e-5
@@ -62,3 +63,31 @@ def test_topk_reference_matches_the_cpu_port():
     np.testing.assert_array_equal(ref_topk(s, 7), [0, 3, 1, 4, 5, 6, 2])
     np.testing.assert_array_equal(ref_topk(s, 3), [5, 6, 2])
     assert len(ref_topk(s, 0)) == 0 and len(ref_topk(s, 9)) == 7
+
+
+@pytest.mark.parametrize("width,qk_scale", [(1, 1.0), (3, 1.0), (5, 0.0), (7, 0.5), (7, -1.0), (9, 3.0), (31, -0.0)],
+                         ids=str)
+def test_fp64_capture_matches_the_cpu_port(width, qk_scale):
+    """The capture reference: logits against the hooked cross-attention of the restated model (capture_logits,
+    timing.py:48-63, SDPA off), maps against filtered_softmax (trim, median with reflect padding inside the row, identity
+    for rows of at most width // 2 frames, scale, softmax) -- on the fp32 logits within fp32 rounding, on the float64
+    logits to float64 rounding."""
+    from oracle import ref_path
+    from whisper.model import MultiHeadAttention, disable_sdpa
+
+    n_heads = 2
+    attn = MultiHeadAttention(64 * n_heads, n_heads)
+    g = torch.Generator().manual_seed(width)
+    for T, F in [(1, 1), (3, width // 2), (5, width // 2 + 1), (9, 40), (4, 300)]:
+        if F < 1:
+            continue
+        q = torch.randn(1, T, 64 * n_heads, generator=g) * 2
+        k = torch.randn(1, F + 5, 64 * n_heads, generator=g)
+        with disable_sdpa():
+            _, qk = attn.qkv_attention(q, k, torch.zeros_like(k))
+        np.testing.assert_allclose(ref_logits(q[0], k[0]).numpy(), qk[0].double().numpy(), rtol=1e-5, atol=1e-5)
+        want = ref_capture(q[0], k[0, :F], width, qk_scale)
+        np.testing.assert_allclose(want.numpy(), ref_path.filtered_softmax(qk[0], F, width, qk_scale).double().numpy(),
+                                   rtol=1e-4, atol=1e-7)
+        port64 = ref_path.filtered_softmax(ref_logits(q[0], k[0]), F, width, qk_scale)
+        np.testing.assert_allclose(want.numpy(), port64.numpy(), rtol=1e-12, atol=0)

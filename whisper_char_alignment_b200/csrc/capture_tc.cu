@@ -89,7 +89,8 @@ enum Bar {
     kNumBars = kXSum + 2
 };
 constexpr int kOffTmem = kOffBar + kNumBars * 8;
-constexpr int kSmemBytes = kOffTmem + 16;
+constexpr int kOffSink = kOffTmem + 16;  // 16 floats the transposition-tile writes of lanes past the last token row go to
+constexpr int kSmemBytes = kOffSink + 64;
 static_assert(kSmemBytes <= 227 * 1024, "shared memory budget");
 
 // ------------------------------------------------------------------ debug trace (WCA_CAPTURE_TRACE)
@@ -544,9 +545,6 @@ __device__ __forceinline__ bool epilogue_tile(const Geo &g, const KernelArgs &a,
         report_rows = g.row_part != nullptr && rows_live && (csize == 1 || cluster_ctarank() == 0) && copy == 0;
         if (report_rows) row_term = row_ok ? sqrtf(gss) / gsum : 0.f;
         inv_sum = __fdividef(m2 > -INFINITY ? ex2_approx(m2 - gmax) : 0.f, gsum);  // this thread's e values are relative to its own m
-        // lanes past the last token row hold finite values nobody stores; as exact zeros in the transposition tile they also
-        // drop out of the column sums of the head scores without a per-element predicate
-        if (g.col_ss != nullptr && !row_ok) inv_sum = 0.f;
         stamp(tr, seq, kEvEpiXSum);
     }
 
@@ -570,6 +568,15 @@ __device__ __forceinline__ bool epilogue_tile(const Geo &g, const KernelArgs &a,
         // x 2 rows; both rows of an instruction have the same (r >> 1) & 3 = k & 3) are then both conflict-free.
         const int sw = (lane >> 1) & 3;
         float4 *tdst = reinterpret_cast<float4 *>(tile + lane * kTilePitch);
+        // Lanes past the last token row computed their values from the Q rows behind the utterance's last token, which a
+        // caller may leave as NaN or inf (and 0 * NaN is NaN): they zero their row of the transposition tile once and send
+        // their block writes to a sink, so that the column sums of the head scores only see token rows (a per-block
+        // predicate or select on those writes cost 2-6 % of the kernel)
+        if (!row_ok) {
+#pragma unroll
+            for (int i = 0; i < 4; ++i) tdst[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+            tdst = reinterpret_cast<float4 *>(smem + kOffSink);
+        }
         const float *tsrc[4];
 #pragma unroll
         for (int j = 0; j < 4; ++j) tsrc[j] = tile + rsel * kTilePitch + 4 * ((c >> 2) ^ j) + (c & 3);

@@ -182,6 +182,23 @@ WCA_API int wca_topk_heads(const float *d_scores, const wca_utt_t *d_utts, int n
 WCA_API int wca_aggregate_heads(const float *d_ws, const int32_t *d_sel, const wca_utt_t *d_utts, int n_utts,
                         int max_tokens, int max_frames, int max_sel, float *d_matrix, wca_stream_t stream);
 
+/* (3d) Std-normalisation of a head list + mean over it: the stock-Whisper baseline, default_find_alignment
+ * (timing.py:156-163).  For every utterance and every i < n_sel of its list d_sel + sel_off, with
+ * a = d_ws + ws_off + d_sel[sel_off + i] * T * F of shape (T, F):
+ *   mu[f] = (1/T) sum_t a[t,f],   sd[f] = sqrt((1/T) sum_t (a[t,f] - mu[f])^2)   over ALL T rows (unbiased=False, :160)
+ *   w_i[t,f] = (a[t,f] - mu[f]) / sd[f]                                            true division: 0/0 is NaN (:161)
+ *   matrix[t - row_begin, f] = (1/n_sel) sum_i w_i[t,f]    heads in list order, rows [row_begin, row_end) (:163, :165)
+ * The mean and the spread are two passes over the column (no one-pass sum of squares), in a fixed order: the result
+ * depends neither on the batch nor on the launch.  w_i goes to d_weights + d_weights_off[u] + i*T*F, laid out
+ * (n_sel, T, F) per utterance (the `weights` default_find_alignment returns); d_weights == NULL (then also
+ * d_weights_off == NULL) skips it and leaves the matrix bit for bit the same.  d_weights_off: n_utts int64 in DEVICE
+ * memory.  Several utterances may share one list (equal sel_off).  n_tokens <= max_tokens <= 448 (Whisper's text
+ * context; a larger max_tokens is WCA_ERR_UNSUPPORTED); a descriptor with n_tokens outside [1, max_tokens], n_sel < 1
+ * or a row range outside [0, n_tokens] fails the launch. */
+WCA_API int wca_normalize_heads(const float *d_ws, const int32_t *d_sel, const wca_utt_t *d_utts, int n_utts,
+                        int max_tokens, int max_frames, float *d_weights, const int64_t *d_weights_off, float *d_matrix,
+                        wca_stream_t stream);
+
 /* (4) Batched DTW + backtrace + boundary extraction.  Replaces timing.py:103
  * `dtw(-matrix)` (upstream dtw_cpu + backtrace), timing.py:110-111 (jump frames) and
  * timing.py:111-113 (start/end times).  One problem per utterance: cost = -matrix

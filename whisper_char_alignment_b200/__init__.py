@@ -11,7 +11,7 @@ Layout
     tokenizer.py     offline stand-in tokenizer
 """
 from .timing import (  # noqa: F401
-    default_find_alignment, dtw, dtw_batch, filter_attention, force_align, force_align_batch, get_attentions, get_attentions_batch,
+    default_find_alignment, default_find_alignment_batch, dtw, dtw_batch, filter_attention, force_align, force_align_batch, get_attentions, get_attentions_batch,
     median_filter_softmax,
 )
 

@@ -24,7 +24,7 @@ ABI_VERSION = 5
 
 EXPORTS = (
     "wca_abi_version", "wca_last_error", "wca_launch_count", "wca_device_info", "wca_capture_attention", "wca_full_attention", "wca_causal_attention", "wca_add_layernorm", "wca_debug_enc_attn_buffer", "wca_debug_capture_trace", "wca_medfilt_softmax",
-    "wca_head_scores", "wca_head_scores_from_partials", "wca_capture_writes_partials", "wca_capture_partials_floats", "wca_topk_heads", "wca_aggregate_heads", "wca_dtw_workspace_bytes", "wca_dtw_align",
+    "wca_head_scores", "wca_head_scores_from_partials", "wca_capture_writes_partials", "wca_capture_partials_floats", "wca_topk_heads", "wca_aggregate_heads", "wca_normalize_heads", "wca_dtw_workspace_bytes", "wca_dtw_align",
 )
 
 
@@ -85,6 +85,7 @@ def load() -> ctypes.CDLL:
     lib.wca_head_scores.argtypes = [vp, vp, i32, i32, i32, i32, f32, f32, f32, vp, vp]
     lib.wca_topk_heads.argtypes = [vp, vp, i32, i32, vp, vp, vp]
     lib.wca_aggregate_heads.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp, vp]
+    lib.wca_normalize_heads.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp, vp, vp]
     lib.wca_dtw_workspace_bytes.restype = i64
     lib.wca_dtw_workspace_bytes.argtypes = [i32, i32, i32]
     lib.wca_dtw_align.argtypes = [vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, i64, vp]
@@ -353,6 +354,20 @@ def aggregate_heads(ws_base: int, sel, d_utts, n_utts, max_tokens, max_frames, m
             load().wca_aggregate_heads(ws_base, _dev_ptr(sel, torch.int32, "sel"), _dev_ptr(d_utts), n_utts, max_tokens,
                                        max_frames, max(int(max_sel), 1), _dev_ptr(matrix, torch.float32, "matrix"), _stream()),
             "wca_aggregate_heads",
+        )
+
+
+def normalize_heads(ws_base: int, sel, d_utts, n_utts, max_tokens, max_frames, matrix, weights=None, weights_off=None):
+    """Std-normalised head maps (`weights` + `weights_off`, both or neither) and their mean (`matrix`)."""
+    if (weights is None) != (weights_off is None):
+        raise WcaError("normalize_heads: give weights and weights_off together or neither")
+    with _timed("wca_normalize_heads"):
+        _check(
+            load().wca_normalize_heads(ws_base, _dev_ptr(sel, torch.int32, "sel"), _dev_ptr(d_utts), n_utts, max_tokens,
+                                       max_frames, _dev_ptr(weights, torch.float32, "weights"),
+                                       _dev_ptr(weights_off, torch.int64, "weights_off"),
+                                       _dev_ptr(matrix, torch.float32, "matrix"), _stream()),
+            "wca_normalize_heads",
         )
 
 

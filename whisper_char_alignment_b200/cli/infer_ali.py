@@ -2,7 +2,7 @@
 
 Flags are the reference's (infer_ali.py:151-173) plus `--dataset synthetic`, `--batch_size` and
 multi-GPU sharding under torchrun.  Per batch the hot path is two calls
-(get_attentions_batch + force_align_batch).  Ranks own cost-balanced shards (sharding.shard_by_cost over the
+(get_attentions_batch + force_align_batch), or one (default_find_alignment_batch) with --default_whisper_timing.  Ranks own cost-balanced shards (sharding.shard_by_cost over the
 datasets' size hints), align them in length-bucketed batches (batching.plan_batches, with the reference's skip
 rule for over-long inputs) and meet once, at the end."""
 from __future__ import annotations
@@ -88,8 +88,8 @@ def _align_batch(args, items, model, tokenizer, qk_scale, local_alignments, pred
     """One length-bucketed batch through the hot path; returns (corrects, predicted, reference) boundary counts."""
     corrects = total_preds = total_gts = 0
     if args.default_whisper_timing:
-        outs = [timing.default_find_alignment(model, tokenizer, it["text_tokens"], it["mel"], it["max_frames"])
-                for _, it in items]
+        outs = timing.default_find_alignment_batch(model, tokenizer, [it["text_tokens"] for _, it in items],
+                                                   [it["mel"] for _, it in items], [it["max_frames"] for _, it in items])
     else:
         maps, _ = timing.get_attentions_batch([it["mel"] for _, it in items], [it["tokens"] for _, it in items], model,
                                               tokenizer, [it["max_frames"] for _, it in items], args.medfilt_width,

@@ -50,6 +50,8 @@ int launch_medfilt_softmax_batched(float *, const wca_utt_t *, int, int, int, in
 int launch_head_scores(const float *, const wca_utt_t *, int, int, int, float, float, float, float *, cudaStream_t);
 int launch_topk_heads(const float *, const wca_utt_t *, int, int, int32_t *, float *, cudaStream_t);
 int launch_aggregate_heads(const float *, const int32_t *, const wca_utt_t *, int, int, int, int, float *, cudaStream_t);
+int launch_normalize_heads(const float *, const int32_t *, const wca_utt_t *, int, int, int, float *, const int64_t *, float *,
+                           cudaStream_t);
 int64_t dtw_workspace_bytes(int, int, int);
 int launch_dtw_align(const float *, const wca_utt_t *, int, int, int, int, int32_t *, int32_t *, int32_t *, int32_t *,
                      const int32_t *, double *, double *, void *, int64_t, cudaStream_t);
@@ -262,6 +264,20 @@ int wca_aggregate_heads(const float *d_ws, const int32_t *d_sel, const wca_utt_t
                   "wca_aggregate_heads: bad geometry");
     if (n_utts == 0) return WCA_OK;
     return launch_aggregate_heads(d_ws, d_sel, d_utts, n_utts, max_tokens, max_frames, max_sel, d_matrix,
+                                  static_cast<cudaStream_t>(stream));
+}
+
+int wca_normalize_heads(const float *d_ws, const int32_t *d_sel, const wca_utt_t *d_utts, int n_utts, int max_tokens,
+                        int max_frames, float *d_weights, const int64_t *d_weights_off, float *d_matrix,
+                        wca_stream_t stream) {
+    WCA_CHECK_ARG(d_ws && d_sel && d_utts && d_matrix, "wca_normalize_heads: null pointer");
+    WCA_CHECK_ARG((d_weights == nullptr) == (d_weights_off == nullptr),
+                  "wca_normalize_heads: give d_weights and d_weights_off together or neither");
+    WCA_CHECK_ARG(n_utts >= 0 && n_utts <= 65535 && max_tokens >= 1 && max_frames >= 1 && max_frames <= 65535 * 32,
+                  "wca_normalize_heads: bad geometry (%d utts, max_tokens %d, max_frames %d)", n_utts, max_tokens,
+                  max_frames);
+    if (n_utts == 0) return WCA_OK;
+    return launch_normalize_heads(d_ws, d_sel, d_utts, n_utts, max_tokens, max_frames, d_weights, d_weights_off, d_matrix,
                                   static_cast<cudaStream_t>(stream));
 }
 

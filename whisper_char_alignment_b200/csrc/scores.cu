@@ -2,7 +2,9 @@
 // Replaces the reference's filter_attention (timing.py:13-43, a Python loop with one
 // blocking .item() per head), coverage_penalty (metrics.py:99-111) and the aggregation
 // branches of force_align (timing.py:84-97).  Everything stays on the device: scores ->
-// ranks -> selected list -> (N, F) matrix, no host round trip in between.
+// ranks -> selected list -> (N, F) matrix, no host round trip in between.  Also the
+// std-normalisation + mean over the alignment heads of the stock-Whisper baseline
+// (default_find_alignment, timing.py:156-163).
 #include "common.cuh"
 
 namespace wca {
@@ -278,6 +280,116 @@ __global__ void __launch_bounds__(256) aggregate_heads_kernel(const float *__res
             matrix[u.matrix_off + (int64_t)(t - u.row_begin) * F + f] = acc_s[t * kWarp + lane] / count;
 }
 
+// Std-normalisation of the alignment heads + mean over heads: the stock-Whisper baseline (timing.py:156-163).
+// grid (ceil(max_frames/32), n_utts), block 256 = 8 warps x 32 columns, dynamic smem T*32 floats of accumulators.
+// Heads are taken 8 at a time.  Statistics: warp g owns head i0 + g and its lanes walk their whole column (lane <-> frame,
+// 128-byte coalesced rows) twice, first for the mean, then for the squared deviations from it; each pass keeps 8
+// partial sums (rows t mod 8, independent add chains) combined in a fixed order, so the result depends on nothing but
+// the column.  The mean is taken of the shifted values a[t,f] - a[0,f]: exact for a constant column (sd = 0, so 0/0
+// gives NaN as in torch) and free of the cancellation of a large mean over a small spread.  Normalisation: warps walk
+// the rows of the group's columns (re-reads come from L1/L2) and add the group's heads, in list order, into the
+// shared accumulators.
+constexpr int kNormGroup = 8;             // heads whose statistics one round computes (one per warp)
+constexpr int kNormMaxTokens = 448;       // Whisper's n_text_ctx: 56 KB of accumulators
+__global__ void __launch_bounds__(256) normalize_heads_kernel(const float *__restrict__ ws,
+                                                              const int32_t *__restrict__ sel,
+                                                              const wca_utt_t *__restrict__ utts, int max_tokens,
+                                                              float *__restrict__ weights,
+                                                              const int64_t *__restrict__ weights_off,
+                                                              float *__restrict__ matrix) {
+    extern __shared__ float acc_s[];  // [T][32]
+    __shared__ float stat[2][2][kNormGroup][kWarp];  // [buffer][mean, sd][head of the group][lane]
+    const wca_utt_t u = utts[blockIdx.y];
+    const int T = u.n_tokens, F = u.n_frames;
+    // a descriptor the accumulators cannot hold, or with no head / a row range outside [0, T): a launch failure,
+    // never a silently wrong matrix
+    if (T < 1 || T > max_tokens || u.n_sel < 1 || u.row_begin < 0 || u.row_end < u.row_begin || u.row_end > T) __trap();
+    const int f0 = blockIdx.x * kWarp;
+    if (f0 >= F) return;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, warps = blockDim.x >> 5;
+    const int f = f0 + lane;
+    const bool live = f < F;
+    const int64_t plane = (int64_t)T * F;
+    float *w_out = weights ? weights + weights_off[blockIdx.y] : nullptr;
+
+    for (int t = warp; t < T; t += warps) acc_s[t * kWarp + lane] = 0.f;
+
+    int buf = 0;
+    for (int i0 = 0; i0 < u.n_sel; i0 += kNormGroup, buf ^= 1) {
+        const int ng = min(kNormGroup, u.n_sel - i0);
+        if (warp < ng && live) {
+            const float *a = ws + u.ws_off + (int64_t)sel[u.sel_off + i0 + warp] * plane + f;
+            const float a0 = a[0];
+            float s[8];
+#pragma unroll
+            for (int j = 0; j < 8; ++j) s[j] = 0.f;
+            int t = 0;
+            for (; t + 8 <= T; t += 8) {
+                float p[8];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) p[j] = a[(int64_t)(t + j) * F];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) s[j] += p[j] - a0;
+            }
+#pragma unroll
+            for (int j = 0; j < 8; ++j)
+                if (t + j < T) s[j] += a[(int64_t)(t + j) * F] - a0;
+            const float mean = a0 + (((s[0] + s[1]) + (s[2] + s[3])) + ((s[4] + s[5]) + (s[6] + s[7]))) / (float)T;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) s[j] = 0.f;
+            for (t = 0; t + 8 <= T; t += 8) {
+                float p[8];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) p[j] = a[(int64_t)(t + j) * F] - mean;
+#pragma unroll
+                for (int j = 0; j < 8; ++j) s[j] = fmaf(p[j], p[j], s[j]);
+            }
+#pragma unroll
+            for (int j = 0; j < 8; ++j)
+                if (t + j < T) {
+                    const float d = a[(int64_t)(t + j) * F] - mean;
+                    s[j] = fmaf(d, d, s[j]);
+                }
+            const float var = (((s[0] + s[1]) + (s[2] + s[3])) + ((s[4] + s[5]) + (s[6] + s[7]))) / (float)T;
+            stat[buf][0][warp][lane] = mean;
+            stat[buf][1][warp][lane] = sqrtf(var);  // population std (unbiased=False, timing.py:160)
+        }
+        __syncthreads();  // the statistics of this group; the other buffer is still read by no one
+        if (live) {
+            const float *a[kNormGroup];
+            float mu[kNormGroup], sd[kNormGroup];
+#pragma unroll
+            for (int g = 0; g < kNormGroup; ++g) {
+                const int i = min(i0 + g, u.n_sel - 1);  // past the end: a valid pointer that is never loaded from
+                a[g] = ws + u.ws_off + (int64_t)sel[u.sel_off + i] * plane + f;
+                mu[g] = stat[buf][0][g][lane];
+                sd[g] = stat[buf][1][g][lane];
+            }
+            for (int t = warp; t < T; t += warps) {
+                float acc = acc_s[t * kWarp + lane];
+#pragma unroll
+                for (int g = 0; g < kNormGroup; ++g)
+                    if (g < ng) {
+                        const float w = (a[g][(int64_t)t * F] - mu[g]) / sd[g];  // true division: 0/0 is NaN (timing.py:161)
+                        if (w_out) w_out[(int64_t)(i0 + g) * plane + (int64_t)t * F + f] = w;
+                        acc += w;
+                    }
+                acc_s[t * kWarp + lane] = acc;
+            }
+        }
+        // the next group writes the other statistics buffer, so one barrier per group suffices: a warp that reaches
+        // the next group's barrier has finished reading this group's buffer, and buffer `buf` is only written again
+        // after that barrier
+    }
+
+    // rows are accumulated by warp (t % warps) but written out by warp ((t - row_begin) % warps)
+    __syncthreads();
+    const float count = (float)u.n_sel;  // torch.mean = sum / count (timing.py:163)
+    if (live)
+        for (int t = u.row_begin + warp; t < u.row_end; t += warps)
+            matrix[u.matrix_off + (int64_t)(t - u.row_begin) * F + f] = acc_s[t * kWarp + lane] / count;
+}
+
 int launch_head_scores(const float *d_ws, const wca_utt_t *d_utts, int n_utts, int n_heads, int max_frames, float w_col,
                        float w_row, float w_cov, float *d_scores, cudaStream_t stream) {
     (void)max_frames;  // any row length: the kernel walks it in chunks of 256 columns
@@ -331,6 +443,24 @@ int launch_aggregate_heads(const float *d_ws, const int32_t *d_sel, const wca_ut
         }
         count_launch();
     }
+    return WCA_OK;
+}
+
+int launch_normalize_heads(const float *d_ws, const int32_t *d_sel, const wca_utt_t *d_utts, int n_utts, int max_tokens,
+                           int max_frames, float *d_weights, const int64_t *d_weights_off, float *d_matrix,
+                           cudaStream_t stream) {
+    if (max_tokens > kNormMaxTokens) {
+        set_error("wca_normalize_heads: max_tokens=%d exceeds the %d token rows of the shared-memory accumulator",
+                  max_tokens, kNormMaxTokens);
+        return WCA_ERR_UNSUPPORTED;
+    }
+    const size_t smem = (size_t)max_tokens * kWarp * sizeof(float);
+    // 4 KB of static statistics: from 353 token rows on, the accumulators need the opt-in beyond 48 KB
+    if (smem > 44u * 1024u)
+        WCA_CUDA(cudaFuncSetAttribute(normalize_heads_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const dim3 grid((max_frames + kWarp - 1) / kWarp, n_utts);
+    normalize_heads_kernel<<<grid, 256, smem, stream>>>(d_ws, d_sel, d_utts, max_tokens, d_weights, d_weights_off, d_matrix);
+    WCA_LAUNCH_CHECK("normalize_heads_kernel");
     return WCA_OK;
 }
 

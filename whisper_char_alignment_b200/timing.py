@@ -37,7 +37,8 @@ TOKENS_PER_SECOND = 50  # whisper.audio: SAMPLE_RATE // (HOP_LENGTH * 2)
 
 __all__ = [
     "get_attentions", "get_attentions_batch", "filter_attention", "force_align", "force_align_batch",
-    "dtw", "dtw_batch", "median_filter_softmax", "default_find_alignment", "probe_heads_batch",
+    "dtw", "dtw_batch", "median_filter_softmax", "default_find_alignment", "default_find_alignment_batch",
+    "probe_heads_batch",
 ]
 
 
@@ -221,7 +222,7 @@ def median_filter_softmax(logits: torch.Tensor, max_frames: int, medfilt_width: 
 class _Plan:
     """Offsets of one batch inside the flat work buffers + the uploaded descriptors."""
 
-    def __init__(self, ws_list, row_begin, n_sel_list, word_counts=None):
+    def __init__(self, ws_list, row_begin, n_sel_list, word_counts=None, *, shared_sel=False):
         self.B = B = len(ws_list)
         # head-score partials left by the capture kernel: usable when every utterance carries valid ones in ONE buffer
         parts = [_ScorePartials.of(w) for w in ws_list]
@@ -255,7 +256,7 @@ class _Plan:
         recs["n_sel"], recs["n_words"] = n_sel, n_words
         recs["ws_off"] = delta // 4
         recs["score_off"] = starts(heads)
-        recs["sel_off"] = starts(n_sel)
+        recs["sel_off"] = 0 if shared_sel else starts(n_sel)  # shared_sel: every utterance reads the same head list
         recs["matrix_off"] = starts(n_rows * F)
         recs["path_off"] = starts(n_rows + F)
         recs["jump_off"] = starts(n_rows)
@@ -528,27 +529,83 @@ def _align_single_heads(ws_list, head_lists, tokens_list, tokenizer, aligned_uni
     return out
 
 
+def default_find_alignment_batch(model, tokenizer, text_tokens_list, mels, max_frames_list, *, medfilt_width=7,
+                                 qk_scale=1.0):
+    """The stock-Whisper baseline behind `--default_whisper_timing` (reference timing.py:116-186) for a batch of
+    utterances: only `model.alignment_heads` (:156), std/mean normalisation over tokens (:160-161), mean over heads
+    (:163), DTW (:165), words grouped on spaces.  text_tokens_list: B lists of text tokens; mels: (B, n_mels, n_frames_in)
+    tensor or list of (n_mels, n_frames_in); max_frames_list: B ints.
+    Returns, per utterance, what default_find_alignment returns: (words, start_times, end_times,
+    weights (n_align, T, F) on the device, None), or [[], [], [], [], None] when only EOT remains.
+
+    One capture (get_attentions_batch), one normalisation launch (wca_normalize_heads) and one DTW launch for the
+    whole batch; one device->host copy of the times at the end."""
+    B = len(text_tokens_list)
+    if B == 0:
+        return []
+    if isinstance(mels, (list, tuple)):
+        mels = torch.stack(list(mels))
+    device = mels.device
+    n_heads = model.dims.n_text_head
+    picked = model.alignment_heads.indices().T  # (n, 2) of (layer, head) in the reference's stack order, timing.py:156
+    n_align = int(picked.shape[0])
+    if n_align == 0:
+        raise ValueError("default_find_alignment: the model has no alignment heads")
+    sel = (picked[:, 0] * n_heads + picked[:, 1]).to(device=device, dtype=torch.int32)
+    tokens = [torch.tensor([*tokenizer.sot_sequence, tokenizer.no_timestamps, *t, tokenizer.eot], device=device)
+              for t in text_tokens_list]
+    maps, _ = get_attentions_batch(mels, tokens, model, tokenizer, max_frames_list, medfilt_width, qk_scale)
+
+    # host side: word grouping defines the boundaries the device gathers (timing.py:167-169)
+    words_all, wb_all = [], []
+    for toks in text_tokens_list:
+        words, word_tokens = split_tokens_on_spaces(list(toks) + [tokenizer.eot], tokenizer, "subword")
+        words_all.append((words, word_tokens))
+        wb_all.append(np.pad(np.cumsum([len(t) for t in word_tokens[:-1]]), (1, 0)).astype(np.int32))
+    word_counts = [max(len(wt) - 1, 0) for _, wt in words_all]
+
+    sot_len = len(tokenizer.sot_sequence)
+    plan = _Plan(maps, sot_len, [n_align] * B, word_counts, shared_sel=True)  # rows sot_len .. T-2, timing.py:165
+    T = plan.recs["n_tokens"].astype(np.int64)
+    F = plan.recs["n_frames"].astype(np.int64)
+    w_sizes = n_align * T * F
+    w_off = np.concatenate([[0], np.cumsum(w_sizes)[:-1]]).astype(np.int64)
+    weights = torch.empty(int(w_sizes.sum()), dtype=torch.float32, device=device)
+    d_w_off = torch.from_numpy(w_off).to(device, non_blocking=True)
+    matrix = torch.empty(max(plan.totals["matrix"], 1), dtype=torch.float32, device=device)
+    _cabi.normalize_heads(plan.base_ptr, sel, plan.d_utts, B, plan.max_tokens, plan.max_frames, matrix, weights, d_w_off)
+
+    wb_flat = np.concatenate([
+        np.pad(wb, (0, wc + 1 - len(wb))) if len(wb) < wc + 1 else wb[: wc + 1] for wb, wc in zip(wb_all, word_counts)
+    ]).astype(np.int32)
+    d_wb = torch.from_numpy(wb_flat).to(device, non_blocking=True)
+    times = torch.empty(2, plan.totals["word"], dtype=torch.float64, device=device)
+    trace_bytes = _cabi.dtw_workspace_bytes(B, plan.max_rows, plan.max_frames)
+    trace_ws = torch.empty(trace_bytes, dtype=torch.uint8, device=device) if trace_bytes else None
+    _cabi.dtw_align(matrix.data_ptr(), plan.d_utts, B, plan.max_rows, plan.max_frames, True, word_bounds=d_wb,
+                    start_times=times[0], end_times=times[1], trace_ws=trace_ws)
+    times_h = times.cpu().numpy()  # the only device->host copy of the call
+
+    results = []
+    for b in range(B):
+        words, word_tokens = words_all[b]
+        if len(word_tokens) <= 1:
+            results.append(_SENTINEL())
+            continue
+        wo, W = int(plan.recs[b]["word_off"]), word_counts[b]
+        w = weights[int(w_off[b]): int(w_off[b] + w_sizes[b])].view(n_align, int(T[b]), int(F[b]))
+        results.append((words, times_h[0, wo: wo + W].copy(), times_h[1, wo: wo + W].copy(), w, None))
+    return results
+
+
 def default_find_alignment(model, tokenizer, text_tokens, mel, max_frames, *, medfilt_width=7, qk_scale=1.0):
     """Drop-in for reference timing.py:116-186 (the stock-Whisper baseline behind
     `--default_whisper_timing`): only `model.alignment_heads`, std/mean normalisation over
-    tokens, mean over heads, DTW, words from `tokenizer.split_to_word_tokens`.
+    tokens, mean over heads, DTW, words grouped on spaces.
     Returns (words, start_times, end_times, weights (heads, T, F) on the device, None).
-
-    Capture, filter, softmax, DTW and boundary extraction are the same kernels as the main
-    path; the head gather and the normalisation of the few selected maps are torch ops."""
-    device = mel.device
-    tokens = torch.tensor([*tokenizer.sot_sequence, tokenizer.no_timestamps, *text_tokens, tokenizer.eot], device=device)
-    maps, _ = get_attentions(mel, tokens, model, tokenizer, max_frames, medfilt_width, qk_scale)
-    n_heads = maps.shape[1]
-    picked = model.alignment_heads.indices().T.to(device)  # (n, 2) of (layer, head), timing.py:156
-    weights = maps.flatten(0, 1).index_select(0, picked[:, 0] * n_heads + picked[:, 1])
-    std, mean = torch.std_mean(weights, dim=-2, keepdim=True, unbiased=False)  # timing.py:160-161
-    weights = (weights - mean) / std
-    res = force_align(weights.mean(dim=0), list(text_tokens), tokenizer, "subword", "grad_norm")
-    if isinstance(res, list):
-        return res
-    words, start_times, end_times, _, _ = res
-    return words, start_times, end_times, weights, None
+    A batch of one of default_find_alignment_batch."""
+    return default_find_alignment_batch(model, tokenizer, [text_tokens], mel.unsqueeze(0), [max_frames],
+                                        medfilt_width=medfilt_width, qk_scale=qk_scale)[0]
 
 
 # ---------------------------------------------------------------------------------

@@ -129,6 +129,24 @@ WCA_API int wca_causal_attention(const float *d_q, const float *d_k, const float
                          int n_kv, int n_heads, int head_dim, int64_t ld_q, int64_t ld_k, int64_t ld_v, int64_t ld_out,
                          wca_stream_t stream);
 
+/* (1b'') Single-query attention of one greedy decode step (upstream whisper/model.py
+ * MultiHeadAttention.qkv_attention with a kv_cache): one query row per batch item, every key visible,
+ *     out[b, h*Dh:(h+1)*Dh] = softmax_j(q[b,h,:] . k[b,j,h,:] * Dh^-1/2) . v[b,j,h,:],   j < n_kv,
+ * fp32 on the CUDA cores.  It serves the decoder's self-attention over its cache of positions 0..p (n_kv = p + 1) and
+ * its cross-attention over the encoder rows.  Row b of q / out is at d_q + b*ld_q / d_out + b*ld_out; key j of item b
+ * at d_k + b*batch_stride_k + j*ld_k, value j at d_v + b*batch_stride_v + j*ld_v (a preallocated cache of which n_kv
+ * rows are live, or one layer's column slice of a grouped K/V projection, is read in place); columns [h*Dh, (h+1)*Dh)
+ * belong to head h.  ld_* and the batch strides are multiples of 4 floats, pointers 16-byte aligned; rows at or past
+ * n_kv are never read.  The keys are split into chunks whose partial results go to d_workspace (at least
+ * wca_decode_attention_workspace_bytes(n_batch, n_heads, n_kv) bytes) and are merged in chunk order: the chunks depend
+ * on n_kv only, so a row gives the same bits alone and inside any batch. */
+WCA_API int64_t wca_decode_attention_workspace_bytes(int n_batch, int n_heads, int n_kv);
+WCA_API int wca_decode_attention(const float *d_q, const float *d_k, const float *d_v, float *d_out,
+                                 int n_batch, int n_kv, int n_heads, int head_dim,
+                                 int64_t ld_q, int64_t ld_k, int64_t ld_v, int64_t ld_out,
+                                 int64_t batch_stride_k, int64_t batch_stride_v,
+                                 void *d_workspace, int64_t workspace_bytes, wca_stream_t stream);
+
 /* (1c) Residual add + LayerNorm of the same forward (upstream ResidualAttentionBlock: `x = x + f(ln(x))`,
  * whisper/model.py LayerNorm = fp32 torch layer_norm): y = x + h (skipped when d_h is NULL; written when d_y is
  * not NULL), n = (y - mean(y)) / sqrt(var(y) + eps) * gamma + beta per row, biased variance, fp32.  All

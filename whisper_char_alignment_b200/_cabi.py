@@ -23,7 +23,8 @@ WCA_MAX_LAYERS = 32
 ABI_VERSION = 5
 
 EXPORTS = (
-    "wca_abi_version", "wca_last_error", "wca_launch_count", "wca_device_info", "wca_capture_attention", "wca_full_attention", "wca_causal_attention", "wca_add_layernorm", "wca_debug_enc_attn_buffer", "wca_debug_capture_trace", "wca_medfilt_softmax",
+    "wca_abi_version", "wca_last_error", "wca_launch_count", "wca_device_info", "wca_capture_attention", "wca_full_attention", "wca_causal_attention", "wca_decode_attention_workspace_bytes", "wca_decode_attention",
+    "wca_add_layernorm", "wca_debug_enc_attn_buffer", "wca_debug_capture_trace", "wca_medfilt_softmax",
     "wca_head_scores", "wca_head_scores_from_partials", "wca_capture_writes_partials", "wca_capture_partials_floats", "wca_topk_heads", "wca_aggregate_heads", "wca_normalize_heads", "wca_dtw_workspace_bytes", "wca_dtw_align",
 )
 
@@ -80,6 +81,9 @@ def load() -> ctypes.CDLL:
     lib.wca_head_scores_from_partials.argtypes = [vp, vp, i32, i32, f32, f32, vp, vp]
     lib.wca_full_attention.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i32, i64, i64, i64, i64, vp]
     lib.wca_causal_attention.argtypes = lib.wca_full_attention.argtypes
+    lib.wca_decode_attention_workspace_bytes.restype = i64
+    lib.wca_decode_attention_workspace_bytes.argtypes = [i32, i32, i32]
+    lib.wca_decode_attention.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, i64, i64, i64, i64, i64, i64, vp, i64, vp]
     lib.wca_add_layernorm.argtypes = [vp, vp, vp, vp, vp, vp, i64, i32, f32, vp]
     lib.wca_medfilt_softmax.argtypes = [vp, i64, i64, i32, i32, f32, vp, vp]
     lib.wca_head_scores.argtypes = [vp, vp, i32, i32, i32, i32, f32, f32, f32, vp, vp]
@@ -286,6 +290,49 @@ def full_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, n_heads: i
                                   n_kv, n_heads, width // n_heads, q.stride(1), k.stride(1), v.stride(1), out.stride(1),
                                   _stream()),
             name,
+        )
+    return out
+
+
+def decode_attention_workspace_bytes(n_batch: int, n_heads: int, n_kv: int) -> int:
+    return int(load().wca_decode_attention_workspace_bytes(int(n_batch), int(n_heads), int(n_kv)))
+
+
+def decode_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, n_heads: int, out: torch.Tensor | None = None,
+                     workspace: torch.Tensor | None = None):
+    """q: (batch, n_heads*64), k, v: (batch, n_kv, n_heads*64), fp32 CUDA, last dim contiguous; any row and batch
+    strides (a column slice of a wider projection, the live rows of a preallocated cache).  Returns
+    softmax(q k^T / 8) v per (batch item, head) as (batch, n_heads*64) (wca_decode_attention: one query row per item,
+    every key visible).  workspace: a uint8 CUDA tensor of at least decode_attention_workspace_bytes, allocated when
+    None."""
+    batch, width = q.shape
+    n_kv = k.shape[1]
+    if n_heads < 1 or width % n_heads:
+        raise WcaError(f"decode_attention: width {width} is not a multiple of n_heads={n_heads}")
+    for t, name in ((q, "q"), (k, "k"), (v, "v")):
+        if not t.is_cuda or t.dtype != torch.float32:
+            raise WcaError(f"decode_attention: {name} must be an fp32 CUDA tensor (no CPU fallback exists)")
+        if t.stride(-1) != 1:
+            raise WcaError(f"decode_attention: {name} must have unit stride along the width")
+    for t, name in ((k, "k"), (v, "v")):
+        if tuple(t.shape) != (batch, n_kv, width):
+            raise WcaError(f"decode_attention: {name} must be (batch, n_kv, width) = {(batch, n_kv, width)}, got {tuple(t.shape)}")
+    if out is None:
+        out = torch.empty(batch, width, dtype=torch.float32, device=q.device)
+    if tuple(out.shape) != (batch, width) or out.dtype != torch.float32 or not out.is_cuda or out.stride(-1) != 1:
+        raise WcaError("decode_attention: out must be an fp32 CUDA (batch, width) tensor with unit stride along the width")
+    need = decode_attention_workspace_bytes(batch, n_heads, n_kv)
+    if workspace is None:
+        workspace = torch.empty(need, dtype=torch.uint8, device=q.device)
+    if not workspace.is_cuda or not workspace.is_contiguous():
+        raise WcaError("decode_attention: workspace must be a contiguous CUDA tensor")
+    with _timed("wca_decode_attention"):
+        _check(
+            load().wca_decode_attention(q.data_ptr(), k.data_ptr(), v.data_ptr(), out.data_ptr(), batch, n_kv, n_heads,
+                                        width // n_heads, q.stride(0), k.stride(1), v.stride(1), out.stride(0), k.stride(0),
+                                        v.stride(0), workspace.data_ptr(), workspace.numel() * workspace.element_size(),
+                                        _stream()),
+            "wca_decode_attention",
         )
     return out
 

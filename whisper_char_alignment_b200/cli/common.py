@@ -38,6 +38,8 @@ def load_model_and_tokenizer(name: str, device, qk_gain: float = 4.0):
 
 
 TRANSCRIBE = os.environ.get("WCA_TRANSCRIBE", "reference")  # offline default: align the reference transcript
+#: tokens the built-in greedy decoder may generate per utterance (whisper's DecodingOptions.sample_len default)
+DECODE_TOKENS = 224
 
 
 def transcript_source(whisper_pkg) -> str:
@@ -53,19 +55,41 @@ def transcribe(whisper_pkg, model, mel, reference_text: str, tokenizer=None) -> 
     if whisper_pkg is not None:
         return whisper_pkg.decode(model, mel, whisper_pkg.DecodingOptions(language="en")).text
     if TRANSCRIBE == "greedy" and tokenizer is not None:
-        return tokenizer.decode(whisper_model.greedy_decode(model, mel, tokenizer))
+        return tokenizer.decode(whisper_model.greedy_decode(model, mel, tokenizer, DECODE_TOKENS))
     return reference_text
 
 
 def prepare(record, tokenizer, unit, device, whisper_pkg, model):
     """One dataset record -> dict with tokens and frame count, or None when the reference would skip it
     (infer_ali.py:78-81)."""
-    _, mel, duration, text, starts, ends, fid = record
-    mel = mel.to(device)
+    mel = record[1].to(device)
+    return _item(record, mel, transcribe(whisper_pkg, model, mel, remove_punctuation(record[3]), tokenizer), tokenizer,
+                 unit, device)
+
+
+def prepare_window(records, tokenizer, unit, device, whisper_pkg, model, batch_size):
+    """prepare() for a window of records, in order.  With WCA_TRANSCRIBE=greedy on a CUDA device (and no
+    openai-whisper) the records are transcribed `batch_size` at a time: one encoder pass per chunk, whose output
+    greedy_decode_cached transcribes and each item keeps (`audio_features`, a view of the chunk's output) for its
+    alignment.  Every other mode transcribes record by record, and its items carry no features."""
+    if not (whisper_pkg is None and TRANSCRIBE == "greedy" and torch.device(device).type == "cuda"):
+        return [prepare(r, tokenizer, unit, device, whisper_pkg, model) for r in records]
+    out = []
+    for chunk in batches(records, batch_size):
+        mels = torch.stack([r[1] for r in chunk]).to(device)
+        with torch.no_grad():
+            xa = model.embed_audio(mels)
+        texts = whisper_model.greedy_decode_cached(model, xa, tokenizer, DECODE_TOKENS)
+        out += [_item(r, mels[i], tokenizer.decode(texts[i]), tokenizer, unit, device, xa[i]) for i, r in enumerate(chunk)]
+    return out
+
+
+def _item(record, mel, transcription, tokenizer, unit, device, audio_features=None):
+    _, _, duration, text, starts, ends, fid = record
     text = remove_punctuation(text)
     # an empty transcription stays empty, as in the reference (its `len(transcription) == ''` guard at
     # infer_ali.py:65 never fires): force_align then returns the EOT-only sentinel and 0 predictions
-    transcription = remove_punctuation(transcribe(whisper_pkg, model, mel, text, tokenizer))
+    transcription = remove_punctuation(transcription)
     text_tokens = encode(transcription, tokenizer, unit)
     tokens = torch.tensor([*tokenizer.sot_sequence, tokenizer.no_timestamps, *text_tokens, tokenizer.eot], device=device)
     max_frames = int(duration) // AUDIO_SAMPLES_PER_TOKEN
@@ -73,7 +97,7 @@ def prepare(record, tokenizer, unit, device, whisper_pkg, model):
         print(fid)
         return None
     return dict(mel=mel, tokens=tokens, text_tokens=text_tokens, max_frames=max_frames, text=text, starts=starts,
-                ends=ends, fid=fid)
+                ends=ends, fid=fid, audio_features=audio_features)
 
 
 def batches(items, size):

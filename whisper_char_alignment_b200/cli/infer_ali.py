@@ -69,11 +69,9 @@ def infer_dataset(args):
     # windows of a few batches: every utterance of a window is prepared (transcribed, tokenised), then the window is
     # cut into length-bucketed batches
     for window in common.batches(mine, args.batch_size * 8):
-        prepared = []
-        for n in window:
-            item = common.prepare(dataset[n], tokenizer, args.aligned_unit_type, device, whisper_pkg, model)
-            if item is not None:
-                prepared.append((n, item))
+        items = common.prepare_window([dataset[n] for n in window], tokenizer, args.aligned_unit_type, device, whisper_pkg,
+                                      model, args.batch_size)
+        prepared = [(n, item) for n, item in zip(window, items) if item is not None]
         plan, _ = batching.plan_batches([len(it["tokens"]) for _, it in prepared], [it["max_frames"] for _, it in prepared],
                                         args.batch_size, n_maps=n_maps)
         for chunk in plan:
@@ -87,13 +85,18 @@ def infer_dataset(args):
 def _align_batch(args, items, model, tokenizer, qk_scale, local_alignments, predictions):
     """One length-bucketed batch through the hot path; returns (corrects, predicted, reference) boundary counts."""
     corrects = total_preds = total_gts = 0
+    # the encoder output the transcription step already computed (greedy mode), else the mels
+    features = None
+    if items[0][1]["audio_features"] is not None:
+        features = torch.stack([it["audio_features"] for _, it in items])
+    mels = None if features is not None else [it["mel"] for _, it in items]
     if args.default_whisper_timing:
-        outs = timing.default_find_alignment_batch(model, tokenizer, [it["text_tokens"] for _, it in items],
-                                                   [it["mel"] for _, it in items], [it["max_frames"] for _, it in items])
+        outs = timing.default_find_alignment_batch(model, tokenizer, [it["text_tokens"] for _, it in items], mels,
+                                                   [it["max_frames"] for _, it in items], audio_features=features)
     else:
-        maps, _ = timing.get_attentions_batch([it["mel"] for _, it in items], [it["tokens"] for _, it in items], model,
-                                              tokenizer, [it["max_frames"] for _, it in items], args.medfilt_width,
-                                              qk_scale)
+        maps, _ = timing.get_attentions_batch(mels, [it["tokens"] for _, it in items], model, tokenizer,
+                                              [it["max_frames"] for _, it in items], args.medfilt_width, qk_scale,
+                                              audio_features=features)
         outs = timing.force_align_batch(maps, [it["text_tokens"] for _, it in items], tokenizer,
                                         aligned_unit_type=args.aligned_unit_type, aggregation=args.aggr,
                                         topk=args.topk, w_colnorm=args.w_colnorm, w_rownorm=args.w_rownorm,

@@ -18,6 +18,7 @@ from ..metrics import eval_n1, eval_n1_strict, get_seg_metrics
 from . import common
 
 N_PROBED_HEADS = 360  # probe_oracle.py:83 `filter_attention(w, topk=360)`
+TRANSCRIBE_BATCH = 16  # utterances per greedy transcription batch (common.prepare_window)
 
 
 def parse_args(argv=None):
@@ -47,11 +48,7 @@ def infer_dataset(args):
     model, tokenizer, whisper_pkg, model_source = common.load_model_and_tokenizer(args.model, device)
     dataset = DATASET[args.dataset](args.scp, n_mels=args.n_mels, device=device)
     corrects = total_preds = total_gts = includes_best = n_probed = 0
-    for n in range(len(dataset)):
-        record = dataset[n]
-        if len(record[3].split()) < args.min_words:
-            continue
-        it = common.prepare(record, tokenizer, args.aligned_unit_type, device, whisper_pkg, model)
+    for it in _prepared(dataset, args, tokenizer, device, whisper_pkg, model):
         if it is None:
             continue
         w, _ = timing.get_attentions(it["mel"], it["tokens"], model, tokenizer, it["max_frames"], args.medfilt_width, 1.0)
@@ -90,6 +87,14 @@ def infer_dataset(args):
     common.dump_results(args, {**results, "model_source": model_source,
                                "transcript_source": common.transcript_source(whisper_pkg)})
     return results
+
+
+def _prepared(dataset, args, tokenizer, device, whisper_pkg, model):
+    """The prepared records with at least --min_words reference words, in dataset order (None where skipped)."""
+    for window in common.batches(range(len(dataset)), TRANSCRIBE_BATCH):
+        records = [r for r in (dataset[n] for n in window) if len(r[3].split()) >= args.min_words]
+        yield from common.prepare_window(records, tokenizer, args.aligned_unit_type, device, whisper_pkg, model,
+                                         TRANSCRIBE_BATCH)
 
 
 def main(argv=None):

@@ -59,6 +59,10 @@ int launch_dtw_align(const float *, const wca_utt_t *, int, int, int, int, int32
 int launch_full_attention(const float *, const float *, const float *, float *, int, int, int, int, int64_t, int64_t, int64_t,
                           int64_t, int, cudaStream_t);
 
+int64_t decode_attention_workspace_bytes(int, int, int);
+int launch_decode_attention(const float *, const float *, const float *, float *, int, int, int, int64_t, int64_t, int64_t,
+                            int64_t, int64_t, int64_t, float *, cudaStream_t);
+
 void set_enc_attn_debug_buffer(float *);
 int launch_add_layernorm(const float *, const float *, const float *, const float *, float *, float *, int64_t, int, float,
                          cudaStream_t);
@@ -176,6 +180,39 @@ int wca_causal_attention(const float *d_q, const float *d_k, const float *d_v, f
                          wca_stream_t stream) {
     return attention_entry("wca_causal_attention", d_q, d_k, d_v, d_out, n_batch, n_q, n_kv, n_heads, head_dim, ld_q, ld_k,
                            ld_v, ld_out, 1, stream);
+}
+
+int64_t wca_decode_attention_workspace_bytes(int n_batch, int n_heads, int n_kv) {
+    if (n_batch < 1 || n_heads < 1 || n_kv < 1) return 0;
+    return decode_attention_workspace_bytes(n_batch, n_heads, n_kv);
+}
+
+int wca_decode_attention(const float *d_q, const float *d_k, const float *d_v, float *d_out, int n_batch, int n_kv,
+                         int n_heads, int head_dim, int64_t ld_q, int64_t ld_k, int64_t ld_v, int64_t ld_out,
+                         int64_t batch_stride_k, int64_t batch_stride_v, void *d_workspace, int64_t workspace_bytes,
+                         wca_stream_t stream) {
+    const char *who = "wca_decode_attention";
+    WCA_CHECK_ARG(d_q && d_k && d_v && d_out && d_workspace, "%s: null pointer", who);
+    if (head_dim != kHeadDim) {
+        set_error("%s: head_dim=%d unsupported (every Whisper size uses 64)", who, head_dim);
+        return WCA_ERR_UNSUPPORTED;
+    }
+    WCA_CHECK_ARG(n_batch >= 1 && n_batch <= 65535 && n_heads >= 1 && n_heads <= 65535 && n_kv >= 1 && n_kv < (1 << 24),
+                  "%s: bad geometry (batch %d, n_kv %d, heads %d)", who, n_batch, n_kv, n_heads);
+    const int64_t width = (int64_t)n_heads * head_dim;
+    WCA_CHECK_ARG(ld_q >= width && ld_k >= width && ld_v >= width && ld_out >= width && ld_q % 4 == 0 && ld_k % 4 == 0 &&
+                      ld_v % 4 == 0 && ld_out % 4 == 0,
+                  "%s: leading dimensions must cover H*Dh=%lld and be multiples of 4", who, (long long)width);
+    WCA_CHECK_ARG(batch_stride_k >= 0 && batch_stride_v >= 0 && batch_stride_k % 4 == 0 && batch_stride_v % 4 == 0,
+                  "%s: batch strides (%lld, %lld) must be non-negative multiples of 4", who, (long long)batch_stride_k,
+                  (long long)batch_stride_v);
+    WCA_CHECK_ARG(((uintptr_t)d_q | (uintptr_t)d_k | (uintptr_t)d_v | (uintptr_t)d_out | (uintptr_t)d_workspace) % 16 == 0,
+                  "%s: pointers must be 16-byte aligned", who);
+    const int64_t need = decode_attention_workspace_bytes(n_batch, n_heads, n_kv);
+    WCA_CHECK_ARG(workspace_bytes >= need, "%s: workspace of %lld bytes, %lld needed (wca_decode_attention_workspace_bytes)",
+                  who, (long long)workspace_bytes, (long long)need);
+    return launch_decode_attention(d_q, d_k, d_v, d_out, n_batch, n_kv, n_heads, ld_q, ld_k, ld_v, ld_out, batch_stride_k,
+                                   batch_stride_v, static_cast<float *>(d_workspace), static_cast<cudaStream_t>(stream));
 }
 
 int wca_add_layernorm(const float *d_x, const float *d_h, const float *d_gamma, const float *d_beta, float *d_y, float *d_n,

@@ -117,14 +117,20 @@ class _ScorePartials:
 
 def get_attentions_batch(mels, tokens_list: Sequence[torch.Tensor], model, tokenizer, max_frames_list,
                          medfilt_width: int = 7, qk_scale: float = 1.0, *, raw_logits: bool = False,
-                         force_simt: bool = False):
+                         force_simt: bool = False, audio_features=None):
     """Batched get_attentions.  mels: (B, n_mels, n_frames_in) tensor or list of (n_mels, n_frames_in);
-    tokens_list: B 1-D int64 tensors; max_frames_list: B ints.
+    tokens_list: B 1-D int64 tensors; max_frames_list: B ints.  audio_features: the encoder output of the batch,
+    (B, n_audio_ctx, d), when it has already been computed (e.g. by the transcription step): the encoder is skipped and
+    `mels` may be None.
     Returns ([weights_b (L,H,T_b,F_b) fp32], [logits_b (T_b, V) fp32])."""
-    if isinstance(mels, (list, tuple)):
-        mels = torch.stack(list(mels))
-    B = mels.shape[0]
-    device = mels.device
+    if audio_features is None:
+        if isinstance(mels, (list, tuple)):
+            mels = torch.stack(list(mels))
+        B = mels.shape[0]
+        device = mels.device
+    else:
+        B = audio_features.shape[0]
+        device = audio_features.device
     if device.type != "cuda":
         raise _cabi.WcaError("get_attentions: tensors must be on a CUDA device (no CPU fallback exists)")
     n_layers = model.dims.n_text_layer
@@ -148,10 +154,10 @@ def get_attentions_batch(mels, tokens_list: Sequence[torch.Tensor], model, token
         # the product model hands the projections over itself (its cross-attention K of all layers comes from ONE GEMM,
         # so there is no per-layer `key` module call to hook)
         with torch.no_grad():
-            out_logits, qs, ks = model.forward_with_cross_qk(mels, tok)
+            out_logits, qs, ks = model.forward_with_cross_qk(mels, tok, audio_features=audio_features)
     else:
         with torch.no_grad(), _CrossAttentionTap(model) as tap:
-            out_logits = model(mels, tok)
+            out_logits = model(mels, tok) if audio_features is None else model.decoder(tok, audio_features)
         qs, ks = tap.q, tap.k
     q_layers = [_as_f32_rows(q) for q in qs]
     k_layers = [_as_f32_rows(k) for k in ks]
@@ -530,11 +536,12 @@ def _align_single_heads(ws_list, head_lists, tokens_list, tokenizer, aligned_uni
 
 
 def default_find_alignment_batch(model, tokenizer, text_tokens_list, mels, max_frames_list, *, medfilt_width=7,
-                                 qk_scale=1.0):
+                                 qk_scale=1.0, audio_features=None):
     """The stock-Whisper baseline behind `--default_whisper_timing` (reference timing.py:116-186) for a batch of
     utterances: only `model.alignment_heads` (:156), std/mean normalisation over tokens (:160-161), mean over heads
     (:163), DTW (:165), words grouped on spaces.  text_tokens_list: B lists of text tokens; mels: (B, n_mels, n_frames_in)
-    tensor or list of (n_mels, n_frames_in); max_frames_list: B ints.
+    tensor or list of (n_mels, n_frames_in); max_frames_list: B ints; audio_features: as get_attentions_batch takes it
+    (mels may then be None).
     Returns, per utterance, what default_find_alignment returns: (words, start_times, end_times,
     weights (n_align, T, F) on the device, None), or [[], [], [], [], None] when only EOT remains.
 
@@ -543,9 +550,9 @@ def default_find_alignment_batch(model, tokenizer, text_tokens_list, mels, max_f
     B = len(text_tokens_list)
     if B == 0:
         return []
-    if isinstance(mels, (list, tuple)):
+    if audio_features is None and isinstance(mels, (list, tuple)):
         mels = torch.stack(list(mels))
-    device = mels.device
+    device = mels.device if audio_features is None else audio_features.device
     n_heads = model.dims.n_text_head
     picked = model.alignment_heads.indices().T  # (n, 2) of (layer, head) in the reference's stack order, timing.py:156
     n_align = int(picked.shape[0])
@@ -554,7 +561,8 @@ def default_find_alignment_batch(model, tokenizer, text_tokens_list, mels, max_f
     sel = (picked[:, 0] * n_heads + picked[:, 1]).to(device=device, dtype=torch.int32)
     tokens = [torch.tensor([*tokenizer.sot_sequence, tokenizer.no_timestamps, *t, tokenizer.eot], device=device)
               for t in text_tokens_list]
-    maps, _ = get_attentions_batch(mels, tokens, model, tokenizer, max_frames_list, medfilt_width, qk_scale)
+    maps, _ = get_attentions_batch(mels, tokens, model, tokenizer, max_frames_list, medfilt_width, qk_scale,
+                                   audio_features=audio_features)
 
     # host side: word grouping defines the boundaries the device gathers (timing.py:167-169)
     words_all, wb_all = [], []

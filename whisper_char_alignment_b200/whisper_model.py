@@ -126,9 +126,25 @@ class Attention(nn.Module):
     def _split(self, t):
         return t.unflatten(-1, (self.n_head, -1)).transpose(1, 2)
 
-    def forward(self, x, xa=None, causal: bool = False, kv=None, tap=None):
+    def forward(self, x, xa=None, causal: bool = False, kv=None, tap=None, cache=None, step: bool = False):
         """kv: (k, v) already projected (views into the decoder's all-layer K/V GEMM); tap: list that receives
-        (q, k) of a cross-attention for the capture kernel."""
+        (q, k) of a cross-attention for the capture kernel.  step: one greedy decode step, x holds one new row per batch
+        item and attends on the decode kernel (csrc/decode_attn.cu) -- a cross-attention over `kv`, a self-attention
+        over its cache = (buffer (batch, n_text_ctx, 2d), pos): the row's K and V go to buffer[:, pos] (K then V), the
+        query attends over buffer[:, :pos + 1]."""
+        if step:
+            from . import _cabi
+
+            if cache is not None:
+                buf, pos = cache
+                w, b = self._qkv.get((self.query, self.key, self.value), x.dtype)
+                d = x.shape[-1]
+                qkv = F.linear(x, w, b)  # (batch, 1, 3d)
+                buf[:, pos:pos + 1].copy_(qkv[..., d:])
+                q, k, v = qkv[..., :d], buf[:, :pos + 1, :d], buf[:, :pos + 1, d:]
+            else:
+                q, (k, v) = self.query(x), kv
+            return self.out(_cabi.decode_attention(q[:, 0], k, v, self.n_head).unsqueeze(1)), None
         fused = FUSED_PROJECTIONS and x.is_cuda and not torch.is_grad_enabled()
         if kv is not None:
             q, (k, v) = self.query(x), kv
@@ -184,15 +200,17 @@ class Block(nn.Module):
         self.mlp = nn.Sequential(_Proj(width, 4 * width), nn.GELU(), _Proj(4 * width, width))
         self.mlp_ln = _Norm(width)
 
-    def forward(self, x, xa=None, causal: bool = False, pending=None, kv=None, tap=None):
+    def forward(self, x, xa=None, causal: bool = False, pending=None, kv=None, tap=None, cache=None):
         """Upstream: x += attn(ln(x)); x += cross_attn(ln(x), xa); x += mlp(ln(x)).  Every residual add is
         paired with the LayerNorm that follows it, so the last add of a block is handed to the next one
-        (`pending`): returns (x, h) with the block's output being x + h."""
+        (`pending`): returns (x, h) with the block's output being x + h.  cache: (buffer, pos) of the self-attention's
+        K/V for one greedy decode step (Attention.forward)."""
+        step = cache is not None
         x, n = _add_ln(x, pending, self.attn_ln)
-        h = self.attn(n, causal=causal)[0]
+        h = self.attn(n, causal=causal, cache=cache, step=step)[0]
         if self.cross_attn is not None:
             x, n = _add_ln(x, h, self.cross_attn_ln)
-            h = self.cross_attn(n, xa, kv=kv, tap=tap)[0]
+            h = self.cross_attn(n, xa, kv=kv, tap=tap, step=step)[0]
         x, n = _add_ln(x, h, self.mlp_ln)
         return x, self.mlp(n)
 
@@ -257,14 +275,22 @@ class TextDecoder(nn.Module):
         w, b = self._cross_kv.setdefault((first, count), _FusedWeights()).get(projections, xa.dtype)
         return F.linear(xa, w, b)
 
-    def forward(self, tokens, xa, tap=None):
-        """tap: list that receives (q, k) of every layer's cross-attention (what timing.get_attentions captures)."""
+    def cross_kv_group(self):
+        """Decoder layers per cross_kv GEMM: the largest divisor of the layer count up to CROSS_KV_GROUP (equal groups
+        only: the capture kernel reads every layer's K with ONE row pitch)."""
+        return max(k for k in range(1, max(1, min(CROSS_KV_GROUP, len(self.blocks))) + 1) if len(self.blocks) % k == 0)
+
+    def forward(self, tokens, xa, tap=None, cache=None):
+        """tap: list that receives (q, k) of every layer's cross-attention (what timing.get_attentions captures).
+        cache: a DecodeCache -- one greedy decode step: tokens (batch, 1) is position cache.pos, attention runs over
+        the cached K/V, the step appends its own and advances cache.pos."""
+        if cache is not None:
+            return self._step(tokens, xa, cache)
         x = self.token_embedding(tokens) + self.positional_embedding[: tokens.shape[-1]]
         x = x.to(xa.dtype)
         d = x.shape[-1]
         fused = FUSED_PROJECTIONS and CROSS_KV_GROUP > 0 and xa.is_cuda and not torch.is_grad_enabled()
-        # equal groups only: the capture kernel reads every layer's K with ONE row pitch
-        group = max(k for k in range(1, max(1, min(CROSS_KV_GROUP, len(self.blocks))) + 1) if len(self.blocks) % k == 0)
+        group = self.cross_kv_group()
         kv_group = None
         pending = None
         for l, blk in enumerate(self.blocks):
@@ -275,6 +301,18 @@ class TextDecoder(nn.Module):
                     kv_group = self.cross_kv(xa, l, min(group, len(self.blocks) - l))
                 kv = (kv_group[..., 2 * i * d:(2 * i + 1) * d], kv_group[..., (2 * i + 1) * d:(2 * i + 2) * d])
             x, pending = blk(x, xa, causal=True, pending=pending, kv=kv, tap=tap)
+        x = _add_ln(x, pending, self.ln)[1]
+        return self._vocab_logits(x)
+
+    def _step(self, tokens, xa, cache):
+        pos = cache.pos
+        if tokens.shape[-1] != 1 or pos >= self.positional_embedding.shape[0]:
+            raise ValueError(f"a decode step takes one token per row inside the text context (position {pos})")
+        x = (self.token_embedding(tokens) + self.positional_embedding[pos: pos + 1]).to(xa.dtype)
+        pending = None
+        for l, blk in enumerate(self.blocks):
+            x, pending = blk(x, xa, causal=True, pending=pending, kv=cache.cross[l], cache=(cache.self_kv[l], pos))
+        cache.pos = pos + 1
         x = _add_ln(x, pending, self.ln)[1]
         return self._vocab_logits(x)
 
@@ -292,6 +330,26 @@ class TextDecoder(nn.Module):
             padded[: w.shape[0]] = w.detach()
             self._padded_vocab, self._padded_key = padded, key
         return F.linear(x, self._padded_vocab)[..., : w.shape[0]]
+
+
+class DecodeCache:
+    """K/V state of a cached greedy decode over audio features xa (batch, n_audio_ctx, d), CUDA fp32: the
+    cross-attention K/V of every decoder layer, computed once with the grouped TextDecoder.cross_kv GEMMs (views into
+    them), and per layer a (batch, n_text_ctx, 2d) self-attention cache, K then V, of which positions < pos are filled."""
+
+    def __init__(self, decoder: TextDecoder, xa: torch.Tensor):
+        from . import _cabi
+
+        if not xa.is_cuda or xa.dtype != torch.float32:
+            raise _cabi.WcaError("the cached decoder needs fp32 CUDA audio features (no CPU fallback exists)")
+        n_layers, (n_ctx, d) = len(decoder.blocks), decoder.positional_embedding.shape
+        group = decoder.cross_kv_group()
+        self.cross = []
+        for first in range(0, n_layers, group):
+            kv = decoder.cross_kv(xa, first, group)
+            self.cross += [(kv[..., 2 * i * d:(2 * i + 1) * d], kv[..., (2 * i + 1) * d:(2 * i + 2) * d]) for i in range(group)]
+        self.self_kv = [torch.empty(xa.shape[0], n_ctx, 2 * d, dtype=xa.dtype, device=xa.device) for _ in range(n_layers)]
+        self.pos = 0
 
 
 class Whisper(nn.Module):
@@ -315,13 +373,15 @@ class Whisper(nn.Module):
     def forward(self, mel, tokens):
         return self.decoder(tokens, self.encoder(mel))
 
-    def forward_with_cross_qk(self, mel, tokens):
+    def forward_with_cross_qk(self, mel, tokens, audio_features=None):
         """(logits, [q_l (batch, T, d)], [k_l (batch, n_ctx, d)]): the teacher-forced forward plus the cross-attention
         projections of every decoder layer, as the capture kernel reads them (k_l may be a strided view of the all-layer
         K/V GEMM).  timing.get_attentions uses this when the model offers it; any other module tree (a stock
-        openai-whisper model) is tapped with forward hooks on cross_attn.query / cross_attn.key instead."""
+        openai-whisper model) is tapped with forward hooks on cross_attn.query / cross_attn.key instead.
+        audio_features: the encoder output of `mel`, already computed (mel is then not read)."""
         tap = []
-        logits = self.decoder(tokens, self.encoder(mel), tap=tap)
+        xa = self.encoder(mel) if audio_features is None else audio_features
+        logits = self.decoder(tokens, xa, tap=tap)
         return logits, [q for q, _ in tap], [k for _, k in tap]
 
     @property
@@ -431,6 +491,37 @@ def greedy_decode(model: Whisper, mel: torch.Tensor, tokenizer, max_tokens: int 
     for row in tokens[:, len(prefix):].tolist():
         out.append(row[: row.index(tokenizer.eot)] if tokenizer.eot in row else row)
     return out[0] if single else out
+
+
+@torch.no_grad()
+def greedy_decode_cached(model: Whisper, audio_features: torch.Tensor, tokenizer, max_tokens: int = 224) -> list:
+    """greedy_decode on a KV cache: the same procedure (prefix, limit, last-position logits, ids above EOT masked,
+    first arg-max, finished rows emit EOT, stop when every row is done, cut at the first EOT) over encoder output that is
+    already computed, audio_features (B, n_audio_ctx, d) fp32 CUDA.  The cross-attention K/V of every layer are
+    projected once per call; each step projects one new token per row, appends its K/V to the layer's cache and attends
+    on wca_decode_attention.  The prefix is fed one token per step.  Returns one list of text tokens per row."""
+    dec = model.decoder
+    cache = DecodeCache(dec, audio_features)
+    b = audio_features.shape[0]
+    prefix = [*tokenizer.sot_sequence, tokenizer.no_timestamps]
+    tokens = torch.tensor([prefix] * b, device=audio_features.device)
+    done = torch.zeros(b, dtype=torch.bool, device=audio_features.device)
+    limit = min(max_tokens, model.dims.n_text_ctx - len(prefix) - 1)
+    for p in range(len(prefix) - 1 if limit > 0 else 0):
+        dec(tokens[:, p:p + 1], audio_features, cache=cache)
+    for _ in range(limit):
+        logits = dec(tokens[:, -1:], audio_features, cache=cache)[:, -1]
+        logits[:, tokenizer.eot + 1:] = -float("inf")  # no special tokens / timestamps in the text
+        nxt = logits.argmax(-1)
+        nxt = torch.where(done, torch.full_like(nxt, tokenizer.eot), nxt)
+        tokens = torch.cat([tokens, nxt[:, None]], dim=1)
+        done |= nxt == tokenizer.eot
+        if bool(done.all()):
+            break
+    out = []
+    for row in tokens[:, len(prefix):].tolist():
+        out.append(row[: row.index(tokenizer.eot)] if tokenizer.eot in row else row)
+    return out
 
 
 def save_checkpoint(model: Whisper, path: str):

@@ -217,6 +217,24 @@ WCA_API int wca_normalize_heads(const float *d_ws, const int32_t *d_sel, const w
                         int max_tokens, int max_frames, float *d_weights, const int64_t *d_weights_off, float *d_matrix,
                         wca_stream_t stream);
 
+/* (3e) Token probabilities: the word confidence of upstream whisper.timing.find_alignment,
+ *     sampled_logits = logits[len(tokenizer.sot_sequence):, : tokenizer.eot]
+ *     token_probs = sampled_logits.softmax(dim=-1)
+ *     text_token_probs = token_probs[np.arange(len(text_tokens)), text_tokens].tolist()
+ * p[r] = softmax(row_r[0 : n_cols])[target_r] for r < n_rows  (logits[len(sot):, :eot].softmax(-1)[arange, text_tokens]).
+ * Rows are read in place: d_rows[r] is the DEVICE address of row r's first logit (any 4-byte alignment, any pitch);
+ * columns >= n_cols are never read.  d_rows (n_rows pointers), d_targets (n_rows int32) and d_probs (n_rows floats) are
+ * DEVICE memory.  One CTA per row, fixed-order reductions: a row gives the same bits alone, inside any batch and on a
+ * repeated launch.
+ * torch semantics: any NaN in the row gives NaN; a +inf gives NaN (exp(inf - inf)); an all -inf row gives NaN (0/0);
+ * a -inf target in a finite row gives exactly 0.
+ * Targets live on the device, so the library cannot check them without synchronising: the caller checks
+ * 0 <= target < n_cols on the host before the launch (upstream would raise an IndexError), as the Python binding
+ * (_cabi.token_probs) does.  An out-of-range target that reaches the kernel gives NaN for its row, never a read
+ * outside the row.  WCA_ERR_INVALID for a null pointer, n_rows < 0 or n_cols < 1; n_rows == 0 does nothing. */
+WCA_API int wca_token_probs(const float *const *d_rows, const int32_t *d_targets, int n_rows, int n_cols,
+                            float *d_probs, wca_stream_t stream);
+
 /* (4) Batched DTW + backtrace + boundary extraction.  Replaces timing.py:103
  * `dtw(-matrix)` (upstream dtw_cpu + backtrace), timing.py:110-111 (jump frames) and
  * timing.py:111-113 (start/end times).  One problem per utterance: cost = -matrix

@@ -25,7 +25,7 @@ ABI_VERSION = 5
 EXPORTS = (
     "wca_abi_version", "wca_last_error", "wca_launch_count", "wca_device_info", "wca_capture_attention", "wca_full_attention", "wca_causal_attention", "wca_decode_attention_workspace_bytes", "wca_decode_attention",
     "wca_add_layernorm", "wca_debug_enc_attn_buffer", "wca_debug_capture_trace", "wca_medfilt_softmax",
-    "wca_head_scores", "wca_head_scores_from_partials", "wca_capture_writes_partials", "wca_capture_partials_floats", "wca_topk_heads", "wca_aggregate_heads", "wca_normalize_heads", "wca_dtw_workspace_bytes", "wca_dtw_align",
+    "wca_head_scores", "wca_head_scores_from_partials", "wca_capture_writes_partials", "wca_capture_partials_floats", "wca_topk_heads", "wca_aggregate_heads", "wca_normalize_heads", "wca_token_probs", "wca_dtw_workspace_bytes", "wca_dtw_align",
 )
 
 
@@ -90,6 +90,7 @@ def load() -> ctypes.CDLL:
     lib.wca_topk_heads.argtypes = [vp, vp, i32, i32, vp, vp, vp]
     lib.wca_aggregate_heads.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp, vp]
     lib.wca_normalize_heads.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp, vp, vp]
+    lib.wca_token_probs.argtypes = [vp, vp, i32, i32, vp, vp]
     lib.wca_dtw_workspace_bytes.restype = i64
     lib.wca_dtw_workspace_bytes.argtypes = [i32, i32, i32]
     lib.wca_dtw_align.argtypes = [vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, i64, vp]
@@ -416,6 +417,35 @@ def normalize_heads(ws_base: int, sel, d_utts, n_utts, max_tokens, max_frames, m
                                        _dev_ptr(matrix, torch.float32, "matrix"), _stream()),
             "wca_normalize_heads",
         )
+
+
+def token_probs(row_addrs: np.ndarray, targets: np.ndarray, n_cols: int, probs: torch.Tensor):
+    """probs[r] = softmax(logits at row_addrs[r], columns [0, n_cols))[targets[r]] (wca_token_probs).  row_addrs: host
+    int64 device addresses of fp32 rows (any 4-byte alignment, any pitch); targets: host ints.  The targets are checked
+    here, on the host, before anything is launched (the library cannot read them without synchronising); both arrays go
+    to the device in one copy."""
+    row_addrs = np.ascontiguousarray(row_addrs, dtype=np.int64).reshape(-1)
+    targets = np.asarray(targets).reshape(-1)
+    n = len(row_addrs)
+    if len(targets) != n:
+        raise WcaError(f"wca_token_probs: {n} rows but {len(targets)} targets")
+    if n and (targets.min() < 0 or targets.max() >= n_cols):
+        bad = int(targets[(targets < 0) | (targets >= n_cols)][0])
+        raise WcaError(f"wca_token_probs: target {bad} outside [0, {n_cols})")
+    if n and (row_addrs % 4).any():
+        raise WcaError("wca_token_probs: row addresses must be 4-byte aligned")
+    if not probs.is_cuda or probs.dtype != torch.float32 or not probs.is_contiguous() or probs.numel() < n:
+        raise WcaError(f"wca_token_probs: probs must be a contiguous fp32 CUDA tensor of at least {n} elements")
+    if n == 0:
+        return
+    packed = np.empty(12 * n, dtype=np.uint8)  # n int64 addresses, then n int32 targets
+    packed[: 8 * n] = row_addrs.view(np.uint8)
+    packed[8 * n:] = targets.astype(np.int32).view(np.uint8)
+    host = torch.from_numpy(packed)
+    dev = host.pin_memory().to(probs.device, non_blocking=True)
+    with _timed("wca_token_probs"):
+        _check(load().wca_token_probs(dev.data_ptr(), dev.data_ptr() + 8 * n, n, int(n_cols), probs.data_ptr(), _stream()),
+               "wca_token_probs")
 
 
 def dtw_workspace_bytes(n_utts, max_rows, max_frames) -> int:

@@ -11,6 +11,7 @@ import argparse
 import os
 from collections import defaultdict
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -40,6 +41,10 @@ def parse_args(argv=None):
     p.add_argument("--save_prediction", action="store_true")
     p.add_argument("--default_whisper_timing", action="store_true")
     p.add_argument("--batch_size", type=int, default=16, help="utterances per launch (the reference uses 1)")
+    # absent from the namespace unless given, so that the results JSON (every flag) of a run without it is unchanged
+    p.add_argument("--word_probabilities", action="store_true", default=argparse.SUPPRESS,
+                   help="with --save_prediction, save each predicted word's probability (whisper's word confidence) "
+                        "as probs_hat")
     return p.parse_args(argv)
 
 
@@ -90,18 +95,26 @@ def _align_batch(args, items, model, tokenizer, qk_scale, local_alignments, pred
     if items[0][1]["audio_features"] is not None:
         features = torch.stack([it["audio_features"] for _, it in items])
     mels = None if features is not None else [it["mel"] for _, it in items]
+    with_probs = getattr(args, "word_probabilities", False)
+    word_probs = None  # per utterance, the probabilities of words[:-1] (--word_probabilities)
     if args.default_whisper_timing:
         outs = timing.default_find_alignment_batch(model, tokenizer, [it["text_tokens"] for _, it in items], mels,
-                                                   [it["max_frames"] for _, it in items], audio_features=features)
+                                                   [it["max_frames"] for _, it in items], audio_features=features,
+                                                   word_probabilities=with_probs)
+        if with_probs:
+            word_probs = [np.zeros(0) if isinstance(out, list) else out[4] for out in outs]
     else:
-        maps, _ = timing.get_attentions_batch(mels, [it["tokens"] for _, it in items], model, tokenizer,
-                                              [it["max_frames"] for _, it in items], args.medfilt_width, qk_scale,
-                                              audio_features=features)
+        maps, logits = timing.get_attentions_batch(mels, [it["tokens"] for _, it in items], model, tokenizer,
+                                                   [it["max_frames"] for _, it in items], args.medfilt_width, qk_scale,
+                                                   audio_features=features)
         outs = timing.force_align_batch(maps, [it["text_tokens"] for _, it in items], tokenizer,
                                         aligned_unit_type=args.aligned_unit_type, aggregation=args.aggr,
                                         topk=args.topk, w_colnorm=args.w_colnorm, w_rownorm=args.w_rownorm,
                                         w_coverage=args.w_coverage)
-    for (n, it), out in zip(items, outs):
+        if with_probs:
+            word_probs = [wp for _, wp in timing.word_probabilities_batch(
+                logits, [it["text_tokens"] for _, it in items], tokenizer, args.aligned_unit_type)]
+    for b, ((n, it), out) in enumerate(zip(items, outs)):
         words, start_times, end_times, ws, _scores = out
         if args.plot:
             from ..plot import plot_attn  # matplotlib is optional
@@ -113,6 +126,8 @@ def _align_batch(args, items, model, tokenizer, qk_scale, local_alignments, pred
         if args.save_prediction:
             predictions[n] = dict(starts=it["starts"], ends=it["ends"], texts=it["text"].split(),
                                   starts_hat=start_times, ends_hat=end_times, predwords=words, fids=it["fid"])
+            if word_probs is not None:
+                predictions[n]["probs_hat"] = word_probs[b]
         if not args.strict:
             hit, _ = eval_n1(it["ends"], end_times, args.tolerance)
             total_gts += len(it["ends"])

@@ -52,6 +52,7 @@ int launch_topk_heads(const float *, const wca_utt_t *, int, int, int32_t *, flo
 int launch_aggregate_heads(const float *, const int32_t *, const wca_utt_t *, int, int, int, int, float *, cudaStream_t);
 int launch_normalize_heads(const float *, const int32_t *, const wca_utt_t *, int, int, int, float *, const int64_t *, float *,
                            cudaStream_t);
+int launch_token_probs(const float *const *, const int32_t *, int, int, float *, cudaStream_t);
 int64_t dtw_workspace_bytes(int, int, int);
 int launch_dtw_align(const float *, const wca_utt_t *, int, int, int, int, int32_t *, int32_t *, int32_t *, int32_t *,
                      const int32_t *, double *, double *, void *, int64_t, cudaStream_t);
@@ -316,6 +317,14 @@ int wca_normalize_heads(const float *d_ws, const int32_t *d_sel, const wca_utt_t
     if (n_utts == 0) return WCA_OK;
     return launch_normalize_heads(d_ws, d_sel, d_utts, n_utts, max_tokens, max_frames, d_weights, d_weights_off, d_matrix,
                                   static_cast<cudaStream_t>(stream));
+}
+
+int wca_token_probs(const float *const *d_rows, const int32_t *d_targets, int n_rows, int n_cols, float *d_probs,
+                    wca_stream_t stream) {
+    WCA_CHECK_ARG(d_rows && d_targets && d_probs, "wca_token_probs: null pointer");
+    WCA_CHECK_ARG(n_rows >= 0 && n_cols >= 1, "wca_token_probs: bad shape (%d rows, %d columns)", n_rows, n_cols);
+    if (n_rows == 0) return WCA_OK;
+    return launch_token_probs(d_rows, d_targets, n_rows, n_cols, d_probs, static_cast<cudaStream_t>(stream));
 }
 
 int64_t wca_dtw_workspace_bytes(int n_utts, int max_rows, int max_frames) {

@@ -8,6 +8,8 @@ error behaviour as the reference's timing.py, with the arithmetic on sm_100a ker
     force_align(ws, tokens, tokenizer, aligned_unit_type='subword', aggregation="mean", topk=-1,
                 w_colnorm=1.0, w_rownorm=1.0, w_coverage=0.0)
         reference timing.py:69-114
+    word_probabilities_batch(logits_list, text_tokens_list, tokenizer, aligned_unit_type='subword')
+        the word confidence of upstream whisper.timing.find_alignment, which the reference drops
 
 plus `*_batch` variants that push many utterances through one launch of each kernel
 (the reference is strictly one utterance at a time, infer_ali.py:48,57).
@@ -38,7 +40,7 @@ TOKENS_PER_SECOND = 50  # whisper.audio: SAMPLE_RATE // (HOP_LENGTH * 2)
 __all__ = [
     "get_attentions", "get_attentions_batch", "filter_attention", "force_align", "force_align_batch",
     "dtw", "dtw_batch", "median_filter_softmax", "default_find_alignment", "default_find_alignment_batch",
-    "probe_heads_batch",
+    "probe_heads_batch", "word_probabilities_batch",
 ]
 
 
@@ -535,18 +537,69 @@ def _align_single_heads(ws_list, head_lists, tokens_list, tokenizer, aligned_uni
     return out
 
 
+def word_probabilities_batch(logits_list, text_tokens_list, tokenizer, aligned_unit_type="subword"):
+    """Per-word probabilities of upstream whisper.timing.find_alignment for a batch of utterances:
+        token_probs = logits[len(sot_sequence):, :eot].softmax(-1)[arange(len(text_tokens)), text_tokens]
+        word_probabilities = [mean(token_probs[i:j]) for each word's token range [i, j)]
+    logits_list: per utterance the (T_b, V) fp32 CUDA logits of its teacher-forced tokens
+    [*sot_sequence, no_timestamps, *text_tokens, eot], as get_attentions_batch returns them (read in place, never
+    copied); text_tokens_list: the text tokens.  Words are grouped as force_align groups them
+    (split_tokens_on_spaces(tokens + [eot], tokenizer, aligned_unit_type)), so word i is force_align's words[i]; the
+    EOT word gets no probability.
+    Returns, per utterance, (token_probs float32 (n_text,), word_probs float64 (W,)), the word probabilities the float64
+    mean of their tokens' in token order (np.mean, as upstream).  One wca_token_probs launch and one device->host copy
+    for the whole batch."""
+    B = len(logits_list)
+    if len(text_tokens_list) != B:
+        raise ValueError("logits_list and text_tokens_list must have the same batch length")
+    if B == 0:
+        return []
+    for lg in logits_list:
+        if not lg.is_cuda:
+            raise _cabi.WcaError("word_probabilities: logits must be CUDA tensors (no CPU fallback exists)")
+        if lg.dtype != torch.float32 or lg.dim() != 2 or lg.stride(-1) != 1:
+            raise _cabi.WcaError("word_probabilities: logits must be fp32 (T, V) with unit stride along the vocabulary")
+    sot_len = len(tokenizer.sot_sequence)
+    n_cols = int(tokenizer.eot)  # the text vocabulary, logits[..., :eot]
+    texts = [np.asarray(list(t), dtype=np.int64) for t in text_tokens_list]
+    for lg, t in zip(logits_list, texts):
+        if lg.shape[0] < sot_len + len(t) or lg.shape[1] < n_cols:
+            raise ValueError(f"logits of shape {tuple(lg.shape)} do not cover {len(t)} text tokens after the "
+                             f"{sot_len}-token SOT sequence and {n_cols} text-vocabulary columns")
+    # device address of row sot_len + i of every utterance
+    addrs = np.concatenate([lg.data_ptr() + 4 * lg.stride(0) * (sot_len + np.arange(len(t), dtype=np.int64))
+                            for lg, t in zip(logits_list, texts)])
+    n_rows = len(addrs)
+    probs = torch.empty(max(n_rows, 1), dtype=torch.float32, device=logits_list[0].device)
+    _cabi.token_probs(addrs, np.concatenate(texts), n_cols, probs)
+    probs_h = probs[:n_rows].cpu().numpy()  # the only device->host copy of the call
+
+    out, off = [], 0
+    for toks in texts:
+        tp = probs_h[off: off + len(toks)]
+        off += len(toks)
+        _, word_tokens = split_tokens_on_spaces(toks.tolist() + [tokenizer.eot], tokenizer, aligned_unit_type)
+        wb = np.pad(np.cumsum([len(t) for t in word_tokens[:-1]]), (1, 0))
+        tp64 = tp.astype(np.float64)  # upstream averages the Python floats of .tolist()
+        out.append((tp.copy(), np.array([np.mean(tp64[i:j]) for i, j in zip(wb[:-1], wb[1:])], dtype=np.float64)))
+    return out
+
+
 def default_find_alignment_batch(model, tokenizer, text_tokens_list, mels, max_frames_list, *, medfilt_width=7,
-                                 qk_scale=1.0, audio_features=None):
+                                 qk_scale=1.0, audio_features=None, word_probabilities=False):
     """The stock-Whisper baseline behind `--default_whisper_timing` (reference timing.py:116-186) for a batch of
     utterances: only `model.alignment_heads` (:156), std/mean normalisation over tokens (:160-161), mean over heads
     (:163), DTW (:165), words grouped on spaces.  text_tokens_list: B lists of text tokens; mels: (B, n_mels, n_frames_in)
     tensor or list of (n_mels, n_frames_in); max_frames_list: B ints; audio_features: as get_attentions_batch takes it
     (mels may then be None).
     Returns, per utterance, what default_find_alignment returns: (words, start_times, end_times,
-    weights (n_align, T, F) on the device, None), or [[], [], [], [], None] when only EOT remains.
+    weights (n_align, T, F) on the device, None), or [[], [], [], [], None] when only EOT remains.  With
+    word_probabilities=True the fifth element is the float64 word-probability array of word_probabilities_batch (words
+    grouped with "subword"), where upstream find_alignment carries it; words and times are the same bit for bit.
 
     One capture (get_attentions_batch), one normalisation launch (wca_normalize_heads) and one DTW launch for the
-    whole batch; one device->host copy of the times at the end."""
+    whole batch; one device->host copy of the times at the end (plus one wca_token_probs launch and its copy with
+    word_probabilities=True)."""
     B = len(text_tokens_list)
     if B == 0:
         return []
@@ -561,8 +614,11 @@ def default_find_alignment_batch(model, tokenizer, text_tokens_list, mels, max_f
     sel = (picked[:, 0] * n_heads + picked[:, 1]).to(device=device, dtype=torch.int32)
     tokens = [torch.tensor([*tokenizer.sot_sequence, tokenizer.no_timestamps, *t, tokenizer.eot], device=device)
               for t in text_tokens_list]
-    maps, _ = get_attentions_batch(mels, tokens, model, tokenizer, max_frames_list, medfilt_width, qk_scale,
-                                   audio_features=audio_features)
+    maps, logits = get_attentions_batch(mels, tokens, model, tokenizer, max_frames_list, medfilt_width, qk_scale,
+                                        audio_features=audio_features)
+    word_probs = None
+    if word_probabilities:
+        word_probs = [wp for _, wp in word_probabilities_batch(logits, text_tokens_list, tokenizer, "subword")]
 
     # host side: word grouping defines the boundaries the device gathers (timing.py:167-169)
     words_all, wb_all = [], []
@@ -602,18 +658,21 @@ def default_find_alignment_batch(model, tokenizer, text_tokens_list, mels, max_f
             continue
         wo, W = int(plan.recs[b]["word_off"]), word_counts[b]
         w = weights[int(w_off[b]): int(w_off[b] + w_sizes[b])].view(n_align, int(T[b]), int(F[b]))
-        results.append((words, times_h[0, wo: wo + W].copy(), times_h[1, wo: wo + W].copy(), w, None))
+        results.append((words, times_h[0, wo: wo + W].copy(), times_h[1, wo: wo + W].copy(), w,
+                        None if word_probs is None else word_probs[b]))
     return results
 
 
-def default_find_alignment(model, tokenizer, text_tokens, mel, max_frames, *, medfilt_width=7, qk_scale=1.0):
+def default_find_alignment(model, tokenizer, text_tokens, mel, max_frames, *, medfilt_width=7, qk_scale=1.0,
+                           word_probabilities=False):
     """Drop-in for reference timing.py:116-186 (the stock-Whisper baseline behind
     `--default_whisper_timing`): only `model.alignment_heads`, std/mean normalisation over
     tokens, mean over heads, DTW, words grouped on spaces.
-    Returns (words, start_times, end_times, weights (heads, T, F) on the device, None).
-    A batch of one of default_find_alignment_batch."""
+    Returns (words, start_times, end_times, weights (heads, T, F) on the device, None), the fifth element the word
+    probabilities with word_probabilities=True.  A batch of one of default_find_alignment_batch."""
     return default_find_alignment_batch(model, tokenizer, [text_tokens], mel.unsqueeze(0), [max_frames],
-                                        medfilt_width=medfilt_width, qk_scale=qk_scale)[0]
+                                        medfilt_width=medfilt_width, qk_scale=qk_scale,
+                                        word_probabilities=word_probabilities)[0]
 
 
 # ---------------------------------------------------------------------------------

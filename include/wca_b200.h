@@ -235,6 +235,32 @@ WCA_API int wca_normalize_heads(const float *d_ws, const int32_t *d_sel, const w
 WCA_API int wca_token_probs(const float *const *d_rows, const int32_t *d_targets, int n_rows, int n_cols,
                             float *d_probs, wca_stream_t stream);
 
+/* (3f) Word-boundary hits of many alignments: the hit count of the reference's scoring, metrics.py:22-43 (eval_n1)
+ * and metrics.py:45-72 (eval_n1_strict), one count per problem p < n_problems.
+ *   y_hat = d_end_times[word_off .. word_off + n_words) of d_utts[p] (float64 seconds, read in place where
+ *           wca_dtw_align wrote them with the same descriptors);
+ *   y     = d_ref_times[d_ref_off[u] .. d_ref_off[u + 1]) of the reference list u = d_utt_of[p] (float64).
+ * WCA_HITS_PLAIN  : eval_n1(y, y_hat, tolerance): greedy in-order two-pointer match, |y[i] - y_hat[j]| <= tolerance
+ *                   in double; a pair that orders neither way (NaN) stops the match; an empty y_hat gives 0.
+ * WCA_HITS_STRICT : eval_n1_strict's true positives: for each predicted word i in order, the first unused reference
+ *                   index j with d_ref_ids[d_ref_off[u] + j] == d_hyp_ids[d_hyp_off[u] + i] and
+ *                   |y[j] - y_hat[i]| <= tolerance is taken; NaN never matches.  The ids are the caller's integer
+ *                   codes of the normalised words (w.lower().strip(string.punctuation)); hypothesis ids are per
+ *                   reference list u, since every problem of one utterance has the same words.  A reference list of
+ *                   more than WCA_HITS_MAX_STRICT_REF_WORDS words gives -1 (the caller checks that on the host).
+ * n_pred = n_words and n_ref = d_ref_off[u + 1] - d_ref_off[u] in both modes (eval_n1_strict's tp + fp, tp + fn).
+ * Every array is DEVICE memory: d_utt_of (n_problems int32), d_ref_off (int64, one past the largest u used),
+ * d_hits (n_problems int32); d_ref_ids, d_hyp_ids, d_hyp_off may be NULL in the plain mode.  One warp per problem:
+ * a problem gives the same count alone and inside any batch.  Nothing outside d_hits[0 : n_problems) is written.
+ * WCA_ERR_INVALID for a null pointer, n_problems < 0, a negative or NaN tolerance or an unknown mode. */
+#define WCA_HITS_PLAIN 0
+#define WCA_HITS_STRICT 1
+#define WCA_HITS_MAX_STRICT_REF_WORDS 1024
+WCA_API int wca_boundary_hits(const double *d_end_times, const wca_utt_t *d_utts, const int32_t *d_utt_of, int n_problems,
+                              const double *d_ref_times, const int64_t *d_ref_off, const int32_t *d_ref_ids,
+                              const int32_t *d_hyp_ids, const int64_t *d_hyp_off, double tolerance, int mode,
+                              int32_t *d_hits, wca_stream_t stream);
+
 /* (4) Batched DTW + backtrace + boundary extraction.  Replaces timing.py:103
  * `dtw(-matrix)` (upstream dtw_cpu + backtrace), timing.py:110-111 (jump frames) and
  * timing.py:111-113 (start/end times).  One problem per utterance: cost = -matrix

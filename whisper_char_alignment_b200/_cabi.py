@@ -25,8 +25,11 @@ ABI_VERSION = 5
 EXPORTS = (
     "wca_abi_version", "wca_last_error", "wca_launch_count", "wca_device_info", "wca_capture_attention", "wca_full_attention", "wca_causal_attention", "wca_decode_attention_workspace_bytes", "wca_decode_attention",
     "wca_add_layernorm", "wca_debug_enc_attn_buffer", "wca_debug_capture_trace", "wca_medfilt_softmax",
-    "wca_head_scores", "wca_head_scores_from_partials", "wca_capture_writes_partials", "wca_capture_partials_floats", "wca_topk_heads", "wca_aggregate_heads", "wca_normalize_heads", "wca_token_probs", "wca_dtw_workspace_bytes", "wca_dtw_align",
+    "wca_head_scores", "wca_head_scores_from_partials", "wca_capture_writes_partials", "wca_capture_partials_floats", "wca_topk_heads", "wca_aggregate_heads", "wca_normalize_heads", "wca_token_probs", "wca_boundary_hits", "wca_dtw_workspace_bytes", "wca_dtw_align",
 )
+WCA_HITS_PLAIN = 0
+WCA_HITS_STRICT = 1
+WCA_HITS_MAX_STRICT_REF_WORDS = 1024
 
 
 class WcaError(RuntimeError):
@@ -91,6 +94,7 @@ def load() -> ctypes.CDLL:
     lib.wca_aggregate_heads.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp, vp]
     lib.wca_normalize_heads.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp, vp, vp]
     lib.wca_token_probs.argtypes = [vp, vp, i32, i32, vp, vp]
+    lib.wca_boundary_hits.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp, vp, ctypes.c_double, i32, vp, vp]
     lib.wca_dtw_workspace_bytes.restype = i64
     lib.wca_dtw_workspace_bytes.argtypes = [i32, i32, i32]
     lib.wca_dtw_align.argtypes = [vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, i64, vp]
@@ -446,6 +450,64 @@ def token_probs(row_addrs: np.ndarray, targets: np.ndarray, n_cols: int, probs: 
     with _timed("wca_token_probs"):
         _check(load().wca_token_probs(dev.data_ptr(), dev.data_ptr() + 8 * n, n, int(n_cols), probs.data_ptr(), _stream()),
                "wca_token_probs")
+
+
+def boundary_hits(end_times: torch.Tensor, d_utts: torch.Tensor, utt_of: np.ndarray, ref_times: Sequence[np.ndarray],
+                  tolerance: float, hits: torch.Tensor, ref_ids: Sequence[np.ndarray] | None = None,
+                  hyp_ids: Sequence[np.ndarray] | None = None, n_pred: np.ndarray | None = None):
+    """hits[p] = eval_n1 (ref_ids is None) or eval_n1_strict hit count of problem p (wca_boundary_hits).
+    end_times: the float64 CUDA end times wca_dtw_align wrote for the descriptors d_utts (read in place); utt_of: host
+    ints, the reference list of each problem; ref_times: per reference list, its float64 end times; strict mode:
+    ref_ids / hyp_ids, per reference list, the int32 word ids of its reference words and of its hypothesis words, and
+    n_pred, per problem, the n_words of its descriptor (the kernel reads that many hypothesis ids).
+    Every host array goes to the device in one copy; the lengths of the strict mode are checked here."""
+    utt_of = np.ascontiguousarray(utt_of, dtype=np.int32).reshape(-1)
+    n, n_lists = len(utt_of), len(ref_times)
+    strict = ref_ids is not None
+    if strict != (hyp_ids is not None):
+        raise WcaError("wca_boundary_hits: give ref_ids and hyp_ids together or neither")
+    if n and (utt_of.min() < 0 or utt_of.max() >= n_lists):
+        raise WcaError(f"wca_boundary_hits: a problem's reference list is outside [0, {n_lists})")
+    lens = np.array([len(r) for r in ref_times], dtype=np.int64)
+    if strict:
+        if len(ref_ids) != n_lists or len(hyp_ids) != n_lists or any(len(a) != k for a, k in zip(ref_ids, lens)):
+            raise WcaError("wca_boundary_hits: one reference id per reference word of every list is needed")
+        if n_pred is None or len(n_pred) != n:
+            raise WcaError("wca_boundary_hits: the strict mode needs n_pred, one predicted-word count per problem")
+        hyp_lens = np.array([len(h) for h in hyp_ids], dtype=np.int64)
+        if n and (np.asarray(n_pred, dtype=np.int64) > hyp_lens[utt_of]).any():
+            raise WcaError("wca_boundary_hits: a problem has more predicted words than its list has hypothesis ids")
+        if n_lists and lens.max() > WCA_HITS_MAX_STRICT_REF_WORDS:
+            raise WcaError(f"wca_boundary_hits: the strict mode takes at most {WCA_HITS_MAX_STRICT_REF_WORDS} reference "
+                           f"words per list, got {int(lens.max())}")
+    if not hits.is_cuda or hits.dtype != torch.int32 or not hits.is_contiguous() or hits.numel() < n:
+        raise WcaError(f"wca_boundary_hits: hits must be a contiguous int32 CUDA tensor of at least {n} elements")
+    _dev_ptr(end_times, torch.float64, "end_times")
+    # one pinned buffer, 8-byte aligned sections: ref times, ref offsets, hyp offsets, then int32 problem lists and ids
+    cat = lambda arrs, dt: np.concatenate([np.asarray(a, dtype=dt).reshape(-1) for a in arrs]) if len(arrs) else np.zeros(0, dt)  # noqa: E731
+    ref_off = np.concatenate([[0], np.cumsum(lens)]).astype(np.int64)
+    sections = [cat(ref_times, np.float64), ref_off]
+    if strict:
+        sections += [np.concatenate([[0], np.cumsum(hyp_lens)[:-1]]).astype(np.int64) if n_lists else np.zeros(0, np.int64),
+                     cat(ref_ids, np.int32), cat(hyp_ids, np.int32)]
+    sections.append(utt_of)
+    offs, size = [], 0
+    for a in sections:
+        offs.append(size)
+        size += -(-a.nbytes // 8) * 8
+    packed = np.zeros(max(size, 8), dtype=np.uint8)
+    for a, o in zip(sections, offs):
+        packed[o: o + a.nbytes] = a.view(np.uint8)
+    dev = torch.from_numpy(packed).pin_memory().to(hits.device, non_blocking=True)
+    base = dev.data_ptr()
+    ptr = [base + o for o in offs]
+    ref_times_p, ref_off_p, utt_of_p = ptr[0], ptr[1], ptr[-1]
+    hyp_off_p, ref_ids_p, hyp_ids_p = (ptr[2], ptr[3], ptr[4]) if strict else (None, None, None)
+    with _timed("wca_boundary_hits"):
+        _check(load().wca_boundary_hits(end_times.data_ptr(), _dev_ptr(d_utts), utt_of_p, n, ref_times_p, ref_off_p,
+                                        ref_ids_p, hyp_ids_p, hyp_off_p, float(tolerance),
+                                        WCA_HITS_STRICT if strict else WCA_HITS_PLAIN, hits.data_ptr(), _stream()),
+               "wca_boundary_hits")
 
 
 def dtw_workspace_bytes(n_utts, max_rows, max_frames) -> int:

@@ -13,7 +13,7 @@ import sys
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libwca_b200.so")
-SOURCES = ["cabi.cu", "capture_simt.cu", "capture_tc.cu", "enc_attn.cu", "decode_attn.cu", "layernorm.cu", "medfilt_softmax.cu", "scores.cu", "token_probs.cu", "dtw.cu"]
+SOURCES = ["cabi.cu", "capture_simt.cu", "capture_tc.cu", "enc_attn.cu", "decode_attn.cu", "layernorm.cu", "medfilt_softmax.cu", "scores.cu", "token_probs.cu", "boundary_hits.cu", "dtw.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-std=c++17", "-lineinfo",

@@ -105,11 +105,11 @@ def batches(items, size):
         yield items[i:i + size]
 
 
-def dump_results(args, results: dict):
-    """<output_dir>/<%Y-%m-%d-%H:%M:%S>.json = flags merged with metrics (reference infer_ali.py:139-146)."""
+def dump_results(args, results: dict, suffix: str = ""):
+    """<output_dir>/<%Y-%m-%d-%H:%M:%S><suffix>.json = flags merged with metrics (reference infer_ali.py:139-146)."""
     stamp = datetime.datetime.fromtimestamp(time.time()).strftime("%Y-%m-%d-%H:%M:%S")
     os.makedirs(args.output_dir, exist_ok=True)
-    path = os.path.join(args.output_dir, stamp + ".json")
+    path = os.path.join(args.output_dir, stamp + suffix + ".json")
     with open(path, "w") as f:
         json.dump({**vars(args), **results}, f)
     return path, stamp

@@ -45,7 +45,23 @@ def parse_args(argv=None):
     p.add_argument("--word_probabilities", action="store_true", default=argparse.SUPPRESS,
                    help="with --save_prediction, save each predicted word's probability (whisper's word confidence) "
                         "as probs_hat")
-    return p.parse_args(argv)
+    p.add_argument("--alignment_heads", type=str, default=argparse.SUPPRESS, metavar="DUMP_OR_FILE",
+                   help="with --default_whisper_timing, align on these heads: an upstream alignment-head mask string "
+                        "or a -heads.json file written by find_alignment_heads")
+    args = p.parse_args(argv)
+    if hasattr(args, "alignment_heads") and not args.default_whisper_timing:
+        p.error("--alignment_heads needs --default_whisper_timing (the only path that aligns on the model's heads)")
+    return args
+
+
+def alignment_heads_dump(value: str) -> bytes:
+    """The mask string of --alignment_heads: the value itself, or the `mask` of a -heads.json file."""
+    if os.path.isfile(value):
+        import json
+
+        with open(value) as f:
+            value = json.load(f)["mask"]
+    return value.encode("ascii")
 
 
 def infer_dataset(args):
@@ -56,6 +72,8 @@ def infer_dataset(args):
     if world > 1 and not dist.is_initialized():
         dist.init_process_group("nccl", device_id=device)
     model, tokenizer, whisper_pkg, model_source = common.load_model_and_tokenizer(args.model, device)
+    if hasattr(args, "alignment_heads"):
+        model.set_alignment_heads(alignment_heads_dump(args.alignment_heads))
     dataset = DATASET[args.dataset](args.scp, n_mels=args.n_mels, device=device)
     qk_scale = 1.0
     n_maps = model.dims.n_text_layer * model.dims.n_text_head

@@ -53,6 +53,8 @@ int launch_aggregate_heads(const float *, const int32_t *, const wca_utt_t *, in
 int launch_normalize_heads(const float *, const int32_t *, const wca_utt_t *, int, int, int, float *, const int64_t *, float *,
                            cudaStream_t);
 int launch_token_probs(const float *const *, const int32_t *, int, int, float *, cudaStream_t);
+int launch_boundary_hits(const double *, const wca_utt_t *, const int32_t *, int, const double *, const int64_t *,
+                         const int32_t *, const int32_t *, const int64_t *, double, int, int32_t *, cudaStream_t);
 int64_t dtw_workspace_bytes(int, int, int);
 int launch_dtw_align(const float *, const wca_utt_t *, int, int, int, int, int32_t *, int32_t *, int32_t *, int32_t *,
                      const int32_t *, double *, double *, void *, int64_t, cudaStream_t);
@@ -325,6 +327,22 @@ int wca_token_probs(const float *const *d_rows, const int32_t *d_targets, int n_
     WCA_CHECK_ARG(n_rows >= 0 && n_cols >= 1, "wca_token_probs: bad shape (%d rows, %d columns)", n_rows, n_cols);
     if (n_rows == 0) return WCA_OK;
     return launch_token_probs(d_rows, d_targets, n_rows, n_cols, d_probs, static_cast<cudaStream_t>(stream));
+}
+
+int wca_boundary_hits(const double *d_end_times, const wca_utt_t *d_utts, const int32_t *d_utt_of, int n_problems,
+                      const double *d_ref_times, const int64_t *d_ref_off, const int32_t *d_ref_ids,
+                      const int32_t *d_hyp_ids, const int64_t *d_hyp_off, double tolerance, int mode, int32_t *d_hits,
+                      wca_stream_t stream) {
+    WCA_CHECK_ARG(d_end_times && d_utts && d_utt_of && d_ref_times && d_ref_off && d_hits,
+                  "wca_boundary_hits: null pointer");
+    WCA_CHECK_ARG(mode == WCA_HITS_PLAIN || mode == WCA_HITS_STRICT, "wca_boundary_hits: unknown mode %d", mode);
+    WCA_CHECK_ARG(mode == WCA_HITS_PLAIN || (d_ref_ids && d_hyp_ids && d_hyp_off),
+                  "wca_boundary_hits: null pointer (the strict mode needs the word ids)");
+    WCA_CHECK_ARG(n_problems >= 0, "wca_boundary_hits: n_problems=%d", n_problems);
+    WCA_CHECK_ARG(tolerance >= 0.0, "wca_boundary_hits: tolerance %g must be a non-negative number", tolerance);
+    if (n_problems == 0) return WCA_OK;
+    return launch_boundary_hits(d_end_times, d_utts, d_utt_of, n_problems, d_ref_times, d_ref_off, d_ref_ids, d_hyp_ids,
+                                d_hyp_off, tolerance, mode == WCA_HITS_STRICT, d_hits, static_cast<cudaStream_t>(stream));
 }
 
 int64_t wca_dtw_workspace_bytes(int n_utts, int max_rows, int max_frames) {

@@ -48,14 +48,21 @@ def _comm_device():
     return torch.device("cpu")
 
 
-def gather_counters(corrects: int, total_preds: int, total_gts: int):
-    """Sum of the three metric counters over all ranks (every rank gets the totals)."""
+def sum_over_ranks(counts) -> np.ndarray:
+    """Element-wise sum of an integer array of the same shape on every rank, in ONE collective (every rank gets the
+    totals, as int64)."""
+    local = np.asarray(counts, dtype=np.int64)
     if not dist.is_initialized() or dist.get_world_size() == 1:
-        return int(corrects), int(total_preds), int(total_gts)
-    t = torch.tensor([corrects, total_preds, total_gts], dtype=torch.int64, device=_comm_device())
+        return local.copy()
+    t = torch.from_numpy(np.ascontiguousarray(local).reshape(-1)).to(_comm_device())
     parts = [torch.empty_like(t) for _ in range(dist.get_world_size())]
     dist.all_gather(parts, t)
-    tot = torch.stack(parts).sum(0).cpu().tolist()
+    return torch.stack(parts).sum(0).cpu().numpy().reshape(local.shape)
+
+
+def gather_counters(corrects: int, total_preds: int, total_gts: int):
+    """Sum of the three metric counters over all ranks (every rank gets the totals)."""
+    tot = sum_over_ranks([corrects, total_preds, total_gts]).tolist()
     return int(tot[0]), int(tot[1]), int(tot[2])
 
 

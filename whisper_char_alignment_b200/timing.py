@@ -10,6 +10,9 @@ error behaviour as the reference's timing.py, with the arithmetic on sm_100a ker
         reference timing.py:69-114
     word_probabilities_batch(logits_list, text_tokens_list, tokenizer, aligned_unit_type='subword')
         the word confidence of upstream whisper.timing.find_alignment, which the reference drops
+    head_boundary_counts_batch(ws_list, tokens_list, tokenizer, ref_ends_list, ...)
+        every head's word-boundary hits on its own (reference metrics.py eval_n1 / eval_n1_strict), to find a
+        checkpoint's alignment heads
 
 plus `*_batch` variants that push many utterances through one launch of each kernel
 (the reference is strictly one utterance at a time, infer_ali.py:48,57).
@@ -27,7 +30,8 @@ There is no CPU path here: tensors must be CUDA tensors and the extension must b
 from __future__ import annotations
 
 import os
-from typing import Sequence
+import string
+from typing import NamedTuple, Sequence
 
 import numpy as np
 import torch
@@ -40,7 +44,7 @@ TOKENS_PER_SECOND = 50  # whisper.audio: SAMPLE_RATE // (HOP_LENGTH * 2)
 __all__ = [
     "get_attentions", "get_attentions_batch", "filter_attention", "force_align", "force_align_batch",
     "dtw", "dtw_batch", "median_filter_softmax", "default_find_alignment", "default_find_alignment_batch",
-    "probe_heads_batch", "word_probabilities_batch",
+    "probe_heads_batch", "word_probabilities_batch", "head_boundary_counts_batch", "strict_word_ids",
 ]
 
 
@@ -465,17 +469,61 @@ def probe_heads_batch(ws_list, tokens_list, tokenizer, aligned_unit_type="subwor
 
 def _align_single_heads(ws_list, head_lists, tokens_list, tokenizer, aligned_unit_type, return_matrix):
     """force_align(w[l, h][None, None], tokens, aggregation="mean", topk=1) for every listed head of every utterance
-    (probe_oracle.py:89-90), as ONE aggregation launch and ONE DTW launch.  The descriptors of the P = sum_b len(head_lists[b])
-    single-head problems are built with numpy from the utterances' base offsets (no per-head tensor views: a sweep of
-    32 utterances is 12 288 problems).  Returns, per utterance, the list of what force_align returns per head."""
+    (probe_oracle.py:89-90), as ONE aggregation launch and ONE DTW launch (_launch_single_heads).  Returns, per
+    utterance, the list of what force_align returns per head."""
+    B = len(ws_list)
+    if sum(len(h) for h in head_lists) == 0:
+        return [[] for _ in range(B)]
+    sh = _launch_single_heads(ws_list, head_lists, tokens_list, tokenizer, aligned_unit_type)
+    matrix_h = sh.matrix.cpu() if return_matrix else None
+    times_h = sh.times.cpu().numpy()
+    out, p = [], 0
+    word_off, matrix_off = sh.recs["word_off"], sh.recs["matrix_off"]
+    for b in range(B):
+        words, word_tokens = sh.words_all[b]
+        W, per_head = int(sh.n_words[b]), []
+        for _ in range(int(sh.n_heads[b])):
+            if len(word_tokens) <= 1:
+                per_head.append(_SENTINEL())
+            else:
+                wo = int(word_off[p])
+                m = None
+                if return_matrix:
+                    mo, nr, nf = int(matrix_off[p]), int(sh.n_rows[p]), int(sh.F[b])
+                    m = matrix_h[mo: mo + nr * nf].view(nr, nf)
+                per_head.append((words, times_h[0, wo: wo + W], times_h[1, wo: wo + W], m, None))
+            p += 1
+        out.append(per_head)
+    return out
+
+
+class _SingleHeads(NamedTuple):
+    """What _launch_single_heads leaves on the device and on the host: `times` (2, sum of W+1) float64 start / end times
+    at each problem's word_off, `matrix` the aggregated single-head matrices, `recs` / `d_utts` the P problems'
+    descriptors (utterance b's heads are problems sum(n_heads[:b]) .. in list order), `words_all` per utterance the
+    (words, word_tokens) grouping, `n_words`, `n_heads`, `F` per utterance, `n_rows` per problem."""
+
+    times: torch.Tensor
+    matrix: torch.Tensor
+    recs: np.ndarray
+    d_utts: torch.Tensor
+    words_all: list
+    n_words: np.ndarray
+    n_heads: np.ndarray
+    F: np.ndarray
+    n_rows: np.ndarray
+
+
+def _launch_single_heads(ws_list, head_lists, tokens_list, tokenizer, aligned_unit_type):
+    """The single-head alignments of _align_single_heads, left on the device: ONE aggregation launch and ONE DTW launch
+    for the P = sum_b len(head_lists[b]) >= 1 problems, no copy back.  The descriptors are built with numpy from the
+    utterances' base offsets (no per-head tensor views: a sweep of 32 utterances is 12 288 problems)."""
     B = len(ws_list)
     dev = ws_list[0].device
     base_ptr = ws_list[0].data_ptr()
     sot_len = len(tokenizer.sot_sequence)
     n_heads = np.array([len(h) for h in head_lists], dtype=np.int64)
     P = int(n_heads.sum())
-    if P == 0:
-        return [[] for _ in range(B)]
     words_all, wb_all, n_words = [], [], np.zeros(B, dtype=np.int64)
     for b, toks in enumerate(tokens_list):  # the word grouping is a property of the utterance, not of the head
         words, word_tokens = split_tokens_on_spaces(list(toks) + [tokenizer.eot], tokenizer, aligned_unit_type)
@@ -515,25 +563,89 @@ def _align_single_heads(ws_list, head_lists, tokens_list, tokenizer, aligned_uni
     trace_ws = torch.empty(trace_bytes, dtype=torch.uint8, device=dev) if trace_bytes else None
     _cabi.dtw_align(matrix.data_ptr(), d_utts, P, max_rows, max_frames, True, word_bounds=d_wb, start_times=times[0],
                     end_times=times[1], trace_ws=trace_ws)
-    matrix_h = matrix.cpu() if return_matrix else None
-    times_h = times.cpu().numpy()
+    return _SingleHeads(times=times, matrix=matrix, recs=recs, d_utts=d_utts, words_all=words_all, n_words=n_words,
+                        n_heads=n_heads, F=F, n_rows=n_rows)
+
+
+def strict_word_ids(word_lists):
+    """Per list, int32 ids of its words under eval_n1_strict's normalisation (metrics.py:34-35,
+    `w.lower().strip(string.punctuation)`): two words get the same id exactly when eval_n1_strict compares them equal.
+    Ids are shared by all the lists of one call."""
+    table = {}
+    return [np.array([table.setdefault(w.lower().strip(string.punctuation), len(table)) for w in words], dtype=np.int32)
+            for words in word_lists]
+
+
+def head_boundary_counts_batch(ws_list, tokens_list, tokenizer, ref_ends_list, *, aligned_unit_type="subword",
+                               tolerance=0.02, ref_words_list=None):
+    """Every head's word-boundary accuracy on a batch of utterances: the measurement upstream Whisper chose its
+    alignment heads by.  For head (l, h) of utterance b the alignment is force_align(ws_list[b][l, h][None, None],
+    tokens_list[b], tokenizer, aligned_unit_type, aggregation="mean") (what probe_heads_batch aligns per head; no head
+    scoring is run), scored against ref_ends_list[b] as infer_ali scores it:
+        plain  (ref_words_list None): hits = metrics.eval_n1(ref_ends, end_times, tolerance)[0]
+        strict (ref_words_list[b] the reference words): hits = tp of metrics.eval_n1_strict(ref_ends, end_times,
+               ref_words, " ".join(words[:-1]).split(), tolerance)
+    with n_pred = len(end_times) and n_ref = len(ref_ends).  An EOT-only utterance counts (0, 0, len(ref_ends)).
+    Returns, per utterance, an int64 array (L, H, 3) of (hits, n_pred, n_ref).
+    Strict mode raises IndexError, as eval_n1_strict would index past a list, for an utterance with at least one
+    reference boundary and at least one predicted boundary when it has fewer hypothesis words than predicted boundaries
+    or fewer reference words than reference boundaries.  The check is made once per utterance, before any head is
+    scored, so it is slightly stricter than the reference's loop: that loop reads a missing word only while some
+    reference boundary is still unmatched, so a head whose earlier words already matched every reference boundary
+    escapes it there.
+    All L*H*B alignments take one aggregation and one DTW launch, their scoring one wca_boundary_hits launch that reads
+    the end times where the DTW wrote them; the hits are the only device->host copy."""
+    B = len(ws_list)
+    if len(tokens_list) != B or len(ref_ends_list) != B or (ref_words_list is not None and len(ref_words_list) != B):
+        raise ValueError("ws_list, tokens_list, ref_ends_list (and ref_words_list) must have the same batch length")
+    if B == 0:
+        return []
+    for w in ws_list:
+        if not w.is_cuda:
+            raise _cabi.WcaError("head_boundary_counts: attention maps must be CUDA tensors (no CPU fallback exists)")
+    ws_list = [w if w.is_contiguous() else w.contiguous() for w in ws_list]
+    L, H = int(ws_list[0].shape[0]), int(ws_list[0].shape[1])
+    if any(tuple(w.shape[:2]) != (L, H) for w in ws_list):
+        raise ValueError("all utterances of a batch must have the same (layers, heads)")
+    sh = _launch_single_heads(ws_list, [np.arange(L * H)] * B, tokens_list, tokenizer, aligned_unit_type)
+    return [c.reshape(L, H, 3) for c in _boundary_counts(sh, ref_ends_list, tolerance, ref_words_list)]
+
+
+def _boundary_counts(sh, ref_ends_list, tolerance, ref_words_list):
+    """The scoring half of head_boundary_counts_batch on the single-head alignments `sh` left on the device: per
+    utterance, an int64 (n_heads, 3) array of (hits, n_pred, n_ref).  One wca_boundary_hits launch, one copy back."""
+    B = len(sh.words_all)
+    ref_ends = [np.asarray(r, dtype=np.float64).reshape(-1) for r in ref_ends_list]
+    ref_ids = hyp_ids = None
+    if ref_words_list is not None:
+        hyp_words = []
+        for b, (words, _) in enumerate(sh.words_all):
+            W = int(sh.n_words[b])
+            hyp = " ".join(words[:-1]).split()[:W]  # as the CLIs build them (infer_ali.py _align_batch)
+            # eval_n1_strict reads hyp_words[i] / ref_words[j] only inside its loop over the reference boundaries
+            if W and len(ref_ends[b]) and len(hyp) < W:
+                raise IndexError(f"list index out of range: {len(hyp)} hypothesis words for {W} end times (utterance {b})")
+            if W and len(ref_words_list[b]) < len(ref_ends[b]):
+                raise IndexError(f"list index out of range: {len(ref_words_list[b])} reference words for "
+                                 f"{len(ref_ends[b])} reference boundaries (utterance {b})")
+            hyp_words.append(hyp + [""] * (W - len(hyp)))  # only without reference boundaries: never compared
+        ids = strict_word_ids([list(r)[: len(e)] for r, e in zip(ref_words_list, ref_ends)] + hyp_words)
+        # a reference shorter than its boundaries only gets here without predictions: its missing ids match nothing
+        ref_ids = [np.pad(i, (0, len(e) - len(i)), constant_values=-1) for i, e in zip(ids[:B], ref_ends)]
+        hyp_ids = ids[B:]
+    hits = torch.empty(max(int(sh.n_heads.sum()), 1), dtype=torch.int32, device=sh.times.device)
+    _cabi.boundary_hits(sh.times[1], sh.d_utts, np.repeat(np.arange(B), sh.n_heads), ref_ends, tolerance, hits,
+                        ref_ids=ref_ids, hyp_ids=hyp_ids, n_pred=sh.recs["n_words"])
+    hits_h = hits.cpu().numpy().astype(np.int64)  # the only device->host copy of the call
     out, p = [], 0
-    word_off, matrix_off = recs["word_off"], recs["matrix_off"]
     for b in range(B):
-        words, word_tokens = words_all[b]
-        W, per_head = int(n_words[b]), []
-        for _ in range(int(n_heads[b])):
-            if len(word_tokens) <= 1:
-                per_head.append(_SENTINEL())
-            else:
-                wo = int(word_off[p])
-                m = None
-                if return_matrix:
-                    mo, nr, nf = int(matrix_off[p]), int(n_rows[p]), int(F[b])
-                    m = matrix_h[mo: mo + nr * nf].view(nr, nf)
-                per_head.append((words, times_h[0, wo: wo + W], times_h[1, wo: wo + W], m, None))
-            p += 1
-        out.append(per_head)
+        k = int(sh.n_heads[b])
+        c = np.empty((k, 3), dtype=np.int64)
+        c[:, 0] = hits_h[p: p + k]
+        c[:, 1] = sh.n_words[b]
+        c[:, 2] = len(ref_ends[b])
+        out.append(c)
+        p += k
     return out
 
 

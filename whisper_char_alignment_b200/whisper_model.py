@@ -364,6 +364,14 @@ class Whisper(nn.Module):
         upper[dims.n_text_layer // 2:] = True
         self.register_buffer("alignment_heads", upper.to_sparse(), persistent=False)
 
+    def set_alignment_heads(self, dump):
+        """Replace the alignment heads with the mask of an upstream dump (upstream Whisper.set_alignment_heads:
+        base85 of the gzip-compressed (n_text_layer, n_text_head) bool array; heads.encode_alignment_heads writes it)."""
+        from .heads import decode_alignment_heads
+
+        mask = torch.from_numpy(decode_alignment_heads(dump, self.dims.n_text_layer, self.dims.n_text_head))
+        self.register_buffer("alignment_heads", mask.to_sparse().to(self.alignment_heads.device), persistent=False)
+
     def embed_audio(self, mel):
         return self.encoder(mel)
 

@@ -42,7 +42,7 @@ def host_counts(sh, refs, ref_words, tol):
     times_h = sh.times.cpu().numpy()
     out, p = [], 0
     for b, (words, _) in enumerate(sh.words_all):
-        W, H = int(sh.n_words[b]), int(sh.n_heads[b])
+        W, H = int(sh.n_words[b]), int((sh.utt_of == b).sum())
         hyp = " ".join(words[:-1]).split()
         c = np.empty((H, 3), dtype=np.int64)
         for k in range(H):
@@ -131,9 +131,9 @@ def main(argv=None):
             if args.profile:  # the kernel alone, in a run of its own (the profiler slows the host)
                 device_counts(sh, refs, rw, args.tolerance)
                 k_ms = kernel_ms(sh, refs, rw, args.tolerance, args.kernel_iters)
-                report["workloads"][f"{label}/{mode}"] = dict(utterances=n, problems=int(sh.n_heads.sum()),
+                report["workloads"][f"{label}/{mode}"] = dict(utterances=n, problems=len(sh.utt_of),
                                                               words=int(sh.n_words.sum()), kernel_ms=k_ms)
-                print(f"{label}/{mode}: {int(sh.n_heads.sum())} problems: boundary_hits_kernel {k_ms:.4f} ms", flush=True)
+                print(f"{label}/{mode}: {len(sh.utt_of)} problems: boundary_hits_kernel {k_ms:.4f} ms", flush=True)
                 del maps, sh
                 continue
             for _ in range(2):  # warm-up of every shape and arm
@@ -155,7 +155,7 @@ def main(argv=None):
                 step_host_s.append(s)
                 equal &= all(np.array_equal(x, y) for x, y in zip(a, b))
             med = lambda x: float(np.median(x))  # noqa: E731
-            w = dict(utterances=n, problems=int(sh.n_heads.sum()), words=int(sh.n_words.sum()),
+            w = dict(utterances=n, problems=len(sh.utt_of), words=int(sh.n_words.sum()),
                      ref_words=int(sum(len(r) for r in refs)), hits=int(sum(int(c[:, 0].sum()) for c in a)),
                      device_scoring_s=sorted(dev_s), host_scoring_s=sorted(host_s),
                      host_over_device=med(host_s) / med(dev_s), step_with_device_scoring_s=sorted(step_dev_s),

@@ -13,6 +13,11 @@ error behaviour as the reference's timing.py, with the arithmetic on sm_100a ker
     head_boundary_counts_batch(ws_list, tokens_list, tokenizer, ref_ends_list, ...)
         every head's word-boundary hits on its own (reference metrics.py eval_n1 / eval_n1_strict), to find a
         checkpoint's alignment heads
+    get_attentions_widths_batch(mels, tokens_list, model, tokenizer, max_frames_list, widths, ...)
+        the maps of several median-filter widths from one forward
+    alignment_config_counts_batch(maps_by_width, tokens_list, tokenizer, ref_ends_list, configs, ...)
+        the word-boundary counts of many (width, aggregation, top-k, score weights) configurations in one pass, to tune
+        a checkpoint's alignment settings
 
 plus `*_batch` variants that push many utterances through one launch of each kernel
 (the reference is strictly one utterance at a time, infer_ali.py:48,57).
@@ -45,6 +50,7 @@ __all__ = [
     "get_attentions", "get_attentions_batch", "filter_attention", "force_align", "force_align_batch",
     "dtw", "dtw_batch", "median_filter_softmax", "default_find_alignment", "default_find_alignment_batch",
     "probe_heads_batch", "word_probabilities_batch", "head_boundary_counts_batch", "strict_word_ids",
+    "get_attentions_widths_batch", "alignment_config_counts_batch",
 ]
 
 
@@ -129,6 +135,38 @@ def get_attentions_batch(mels, tokens_list: Sequence[torch.Tensor], model, token
     (B, n_audio_ctx, d), when it has already been computed (e.g. by the transcription step): the encoder is skipped and
     `mels` may be None.
     Returns ([weights_b (L,H,T_b,F_b) fp32], [logits_b (T_b, V) fp32])."""
+    fwd = _cross_qk_forward(mels, tokens_list, model, max_frames_list, audio_features)
+    flags = (_cabi.WCA_CAPTURE_RAW_LOGITS if raw_logits else 0) | (_cabi.WCA_CAPTURE_FORCE_SIMT if force_simt else 0)
+    return _capture(fwd, model.dims.n_text_head, medfilt_width, qk_scale, flags)
+
+
+def get_attentions_widths_batch(mels, tokens_list: Sequence[torch.Tensor], model, tokenizer, max_frames_list, widths,
+                                qk_scale: float = 1.0, *, audio_features=None):
+    """get_attentions_batch for several median-filter widths from ONE forward: the teacher-forced forward runs once and
+    the capture kernel runs once per width on the same Q/K.  Arguments as get_attentions_batch; widths: odd ints.
+    Returns {width: (weights, logits)} in the order of `widths` (a repeated width is captured once), each value what
+    get_attentions_batch(..., medfilt_width=width, qk_scale=qk_scale) returns bit for bit, head-score partials
+    included; the logits are the same tensors for every width."""
+    widths = list(dict.fromkeys(int(w) for w in widths))
+    if not widths:
+        raise ValueError("get_attentions_widths_batch: no median-filter width given")
+    fwd = _cross_qk_forward(mels, tokens_list, model, max_frames_list, audio_features)
+    return {w: _capture(fwd, model.dims.n_text_head, w, qk_scale, 0) for w in widths}
+
+
+class _CrossQK(NamedTuple):
+    """The forward half of get_attentions_batch: every decoder layer's cross-attention Q (B*t_max rows) and K, the
+    logits, the token and frame counts of the batch."""
+
+    q_layers: list
+    k_layers: list
+    logits: torch.Tensor
+    lens: list
+    frames: list
+    t_max: int
+
+
+def _cross_qk_forward(mels, tokens_list, model, max_frames_list, audio_features) -> _CrossQK:
     if audio_features is None:
         if isinstance(mels, (list, tuple)):
             mels = torch.stack(list(mels))
@@ -139,8 +177,6 @@ def get_attentions_batch(mels, tokens_list: Sequence[torch.Tensor], model, token
         device = audio_features.device
     if device.type != "cuda":
         raise _cabi.WcaError("get_attentions: tensors must be on a CUDA device (no CPU fallback exists)")
-    n_layers = model.dims.n_text_layer
-    n_heads = model.dims.n_text_head
     n_ctx = model.dims.n_audio_ctx
     lens = [int(t.shape[0]) for t in tokens_list]
     frames = [int(f) for f in max_frames_list]
@@ -165,10 +201,13 @@ def get_attentions_batch(mels, tokens_list: Sequence[torch.Tensor], model, token
         with torch.no_grad(), _CrossAttentionTap(model) as tap:
             out_logits = model(mels, tok) if audio_features is None else model.decoder(tok, audio_features)
         qs, ks = tap.q, tap.k
-    q_layers = [_as_f32_rows(q) for q in qs]
-    k_layers = [_as_f32_rows(k) for k in ks]
+    return _CrossQK([_as_f32_rows(q) for q in qs], [_as_f32_rows(k) for k in ks], out_logits, lens, frames, t_max)
 
-    flags = (_cabi.WCA_CAPTURE_RAW_LOGITS if raw_logits else 0) | (_cabi.WCA_CAPTURE_FORCE_SIMT if force_simt else 0)
+
+def _capture(fwd: _CrossQK, n_heads, medfilt_width, qk_scale, flags):
+    """The capture half of get_attentions_batch: the maps of one median-filter width from the forward's Q/K."""
+    q_layers, k_layers, out_logits, lens, frames, t_max = fwd
+    B, n_layers, device = len(lens), len(q_layers), q_layers[0].device
     # head-score partials: the capture epilogue holds every map value anyway, so it also leaves sum_t ||p[t,:]||_2 and
     # the column sums of squares behind; force_align / filter_attention then score the heads without reading the maps
     with_partials = SCORE_PARTIALS != "0" and _cabi.capture_writes_partials(max(frames), int(medfilt_width), flags)
@@ -482,14 +521,14 @@ def _align_single_heads(ws_list, head_lists, tokens_list, tokenizer, aligned_uni
     for b in range(B):
         words, word_tokens = sh.words_all[b]
         W, per_head = int(sh.n_words[b]), []
-        for _ in range(int(sh.n_heads[b])):
+        for _ in range(len(head_lists[b])):
             if len(word_tokens) <= 1:
                 per_head.append(_SENTINEL())
             else:
                 wo = int(word_off[p])
                 m = None
                 if return_matrix:
-                    mo, nr, nf = int(matrix_off[p]), int(sh.n_rows[p]), int(sh.F[b])
+                    mo, nr, nf = int(matrix_off[p]), int(sh.n_rows[p]), int(sh.recs["n_frames"][p])
                     m = matrix_h[mo: mo + nr * nf].view(nr, nf)
                 per_head.append((words, times_h[0, wo: wo + W], times_h[1, wo: wo + W], m, None))
             p += 1
@@ -497,11 +536,11 @@ def _align_single_heads(ws_list, head_lists, tokens_list, tokenizer, aligned_uni
     return out
 
 
-class _SingleHeads(NamedTuple):
-    """What _launch_single_heads leaves on the device and on the host: `times` (2, sum of W+1) float64 start / end times
-    at each problem's word_off, `matrix` the aggregated single-head matrices, `recs` / `d_utts` the P problems'
-    descriptors (utterance b's heads are problems sum(n_heads[:b]) .. in list order), `words_all` per utterance the
-    (words, word_tokens) grouping, `n_words`, `n_heads`, `F` per utterance, `n_rows` per problem."""
+class _Problems(NamedTuple):
+    """What _launch_problems leaves on the device and on the host: `times` (2, sum of W+1) float64 start / end times
+    at each problem's word_off, `matrix` the aggregated matrices, `recs` / `d_utts` the P problems' descriptors,
+    `utt_of` the utterance of every problem, `words_all` per utterance the (words, word_tokens) grouping, `n_words` per
+    utterance, `n_rows` per problem."""
 
     times: torch.Tensor
     matrix: torch.Tensor
@@ -509,62 +548,90 @@ class _SingleHeads(NamedTuple):
     d_utts: torch.Tensor
     words_all: list
     n_words: np.ndarray
-    n_heads: np.ndarray
-    F: np.ndarray
+    utt_of: np.ndarray
     n_rows: np.ndarray
 
 
 def _launch_single_heads(ws_list, head_lists, tokens_list, tokenizer, aligned_unit_type):
     """The single-head alignments of _align_single_heads, left on the device: ONE aggregation launch and ONE DTW launch
-    for the P = sum_b len(head_lists[b]) >= 1 problems, no copy back.  The descriptors are built with numpy from the
-    utterances' base offsets (no per-head tensor views: a sweep of 32 utterances is 12 288 problems)."""
+    for the P = sum_b len(head_lists[b]) >= 1 problems, no copy back.  Utterance b's heads are problems
+    sum(len(head_lists[:b])) .. in list order.  The descriptors are built with numpy from the utterances' base offsets
+    (no per-head tensor views: a sweep of 32 utterances is 12 288 problems)."""
     B = len(ws_list)
-    dev = ws_list[0].device
     base_ptr = ws_list[0].data_ptr()
-    sot_len = len(tokenizer.sot_sequence)
     n_heads = np.array([len(h) for h in head_lists], dtype=np.int64)
-    P = int(n_heads.sum())
+    utt_of = np.repeat(np.arange(B), n_heads)
+    shapes = np.array([w.shape[2:] for w in ws_list], dtype=np.int64).reshape(B, 2)
+    off = (np.array([w.data_ptr() for w in ws_list], dtype=np.int64) - base_ptr) // 4
+    head = np.concatenate(head_lists).astype(np.int64)
+    ws_off = off[utt_of] + head * (shapes[:, 0] * shapes[:, 1])[utt_of]  # the block of that head: its head list is [0]
+    P = len(utt_of)
+    sel = torch.zeros(P, dtype=torch.int32, device=ws_list[0].device)
+    return _launch_problems(shapes, [(ws_list, sel, utt_of, ws_off, np.arange(P), np.ones(P, dtype=np.int64))],
+                            tokens_list, tokenizer, aligned_unit_type)
+
+
+def _launch_problems(shapes, groups, tokens_list, tokenizer, aligned_unit_type):
+    """force_align_batch's aggregation and DTW for P >= 1 alignment problems over B utterances, left on the device, no
+    copy back.  Every problem aggregates a list of heads of one utterance's maps (rows len(sot_sequence) .. T-2, the
+    utterance's words); several problems may share an utterance.
+    shapes: (B, 2) ints, (T, F) of every utterance's maps.
+    groups: runs of consecutive problems whose maps and head lists live in the same buffers, one aggregation launch
+    each: (ws_list, sel, utt_of, ws_off, sel_off, n_sel) with ws_list the maps of the run (ws_list[0] the base that the
+    float offsets ws_off count from), sel the int32 device buffer of the head lists, and per problem of the run its
+    utterance, the offset of its maps, the offset and the length of its head list in sel.
+    ONE DTW launch for all P problems."""
+    B = len(tokens_list)
+    dev = groups[0][1].device
+    sot_len = len(tokenizer.sot_sequence)
     words_all, wb_all, n_words = [], [], np.zeros(B, dtype=np.int64)
-    for b, toks in enumerate(tokens_list):  # the word grouping is a property of the utterance, not of the head
+    for b, toks in enumerate(tokens_list):  # the word grouping is a property of the utterance, not of the problem
         words, word_tokens = split_tokens_on_spaces(list(toks) + [tokenizer.eot], tokenizer, aligned_unit_type)
         words_all.append((words, word_tokens))
         n_words[b] = max(len(word_tokens) - 1, 0)
         wb = np.pad(np.cumsum([len(t) for t in word_tokens[:-1]]), (1, 0)).astype(np.int32)
         wb_all.append(np.pad(wb, (0, int(n_words[b]) + 1 - len(wb))) if len(wb) < n_words[b] + 1 else wb[: int(n_words[b]) + 1])
-    T = np.array([w.shape[2] for w in ws_list], dtype=np.int64)
-    F = np.array([w.shape[3] for w in ws_list], dtype=np.int64)
-    off = (np.array([w.data_ptr() for w in ws_list], dtype=np.int64) - base_ptr) // 4
-    rep = lambda a: np.repeat(a, n_heads)  # noqa: E731  (per utterance -> per problem)
-    head = np.concatenate(head_lists)
+    T, F = shapes[:, 0], shapes[:, 1]
+    utt_of = np.concatenate([g[2] for g in groups]).astype(np.int64)
+    P = len(utt_of)
     row_end = np.maximum(T - 1, sot_len)
-    n_rows = rep(row_end - sot_len)
+    n_rows = (row_end - sot_len)[utt_of]
+    Fp, Wp = F[utt_of], n_words[utt_of]
 
     def starts(sizes):  # exclusive prefix sum
         return np.concatenate([[0], np.cumsum(sizes)[:-1]])
 
     recs = np.zeros(P, dtype=_cabi.UTT_DTYPE)
-    recs["n_tokens"], recs["n_frames"] = rep(T), rep(F)
-    recs["row_begin"], recs["row_end"] = sot_len, rep(row_end)
-    recs["n_sel"], recs["n_words"] = 1, rep(n_words)
-    recs["ws_off"] = rep(off) + head * rep(T * F)  # the block of that head: its list of selected heads is [0]
-    recs["sel_off"] = np.arange(P)
-    recs["matrix_off"] = starts(n_rows * rep(F))
-    recs["path_off"] = starts(n_rows + rep(F))
+    recs["n_tokens"], recs["n_frames"] = T[utt_of], Fp
+    recs["row_begin"], recs["row_end"] = sot_len, row_end[utt_of]
+    recs["n_words"] = Wp
+    for k, field in ((3, "ws_off"), (4, "sel_off"), (5, "n_sel")):
+        recs[field] = np.concatenate([g[k] for g in groups])
+    recs["matrix_off"] = starts(n_rows * Fp)
+    recs["path_off"] = starts(n_rows + Fp)
     recs["jump_off"] = starts(n_rows)
-    recs["word_off"] = starts(rep(n_words) + 1)
+    recs["word_off"] = starts(Wp + 1)
     d_utts = _cabi.upload_utts(recs, dev)
-    sel = torch.zeros(P, dtype=torch.int32, device=dev)
-    matrix = torch.empty(max(int((n_rows * rep(F)).sum()), 1), dtype=torch.float32, device=dev)
+    matrix = torch.empty(max(int((n_rows * Fp).sum()), 1), dtype=torch.float32, device=dev)
     max_tokens, max_frames, max_rows = int(T.max()), int(F.max()), int(n_rows.max())
-    _cabi.aggregate_heads(base_ptr, sel, d_utts, P, max_tokens, max_frames, matrix, max_sel=1)
-    d_wb = torch.from_numpy(np.concatenate([np.tile(wb_all[b], int(n_heads[b])) for b in range(B)]).astype(np.int32)).to(dev, non_blocking=True)
-    times = torch.empty(2, int((rep(n_words) + 1).sum()), dtype=torch.float64, device=dev)
+    size, p = _cabi.UTT_DTYPE.itemsize, 0
+    for ws_list, sel, u, _, _, n_sel in groups:
+        if len(u):
+            _cabi.aggregate_heads(ws_list[0].data_ptr(), sel, d_utts[p * size: (p + len(u)) * size], len(u), max_tokens,
+                                  max_frames, matrix, max_sel=int(np.max(n_sel)))
+        p += len(u)
+    # every problem's W+1 word bounds at its word_off: gathered from its utterance's bounds
+    wb_cat = np.concatenate(wb_all)
+    wb_start = starts(n_words + 1)
+    idx = np.repeat(wb_start[utt_of] - recs["word_off"], Wp + 1) + np.arange(int((Wp + 1).sum()))
+    d_wb = torch.from_numpy(wb_cat[idx].astype(np.int32)).to(dev, non_blocking=True)
+    times = torch.empty(2, int((Wp + 1).sum()), dtype=torch.float64, device=dev)
     trace_bytes = _cabi.dtw_workspace_bytes(P, max_rows, max_frames)
     trace_ws = torch.empty(trace_bytes, dtype=torch.uint8, device=dev) if trace_bytes else None
     _cabi.dtw_align(matrix.data_ptr(), d_utts, P, max_rows, max_frames, True, word_bounds=d_wb, start_times=times[0],
                     end_times=times[1], trace_ws=trace_ws)
-    return _SingleHeads(times=times, matrix=matrix, recs=recs, d_utts=d_utts, words_all=words_all, n_words=n_words,
-                        n_heads=n_heads, F=F, n_rows=n_rows)
+    return _Problems(times=times, matrix=matrix, recs=recs, d_utts=d_utts, words_all=words_all, n_words=n_words,
+                     utt_of=utt_of, n_rows=n_rows)
 
 
 def strict_word_ids(word_lists):
@@ -611,9 +678,109 @@ def head_boundary_counts_batch(ws_list, tokens_list, tokenizer, ref_ends_list, *
     return [c.reshape(L, H, 3) for c in _boundary_counts(sh, ref_ends_list, tolerance, ref_words_list)]
 
 
+def alignment_config_counts_batch(maps_by_width, tokens_list, tokenizer, ref_ends_list, configs, *,
+                                  aligned_unit_type="subword", tolerance=0.02, ref_words_list=None):
+    """Word-boundary counts of every alignment configuration on a batch of utterances, in one pass over the maps.
+    maps_by_width: {medfilt_width: per utterance its (L, H, T, F) maps} (get_attentions_widths_batch's maps);
+    configs: (medfilt_width, aggr, topk, w_colnorm, w_rownorm, w_coverage) tuples (tuning.Config), aggr "mean" or
+    "topk".  Config c's alignment of utterance b is
+        force_align_batch(maps_by_width[c.medfilt_width], tokens_list, tokenizer, aligned_unit_type, c.aggr, c.topk,
+                          c.w_colnorm, c.w_rownorm, c.w_coverage)[b]
+    scored as infer_ali scores it (eval_n1, or eval_n1_strict with ref_words_list; see head_boundary_counts_batch).
+    Returns, per utterance, an int64 array (len(configs), 3) of (hits, n_pred, n_ref).
+    As in force_align_batch, topk is capped at L*H and topk <= 0 with aggr "topk" raises AssertionError.  An EOT-only
+    utterance counts (0, 0, len(ref_ends)) for every config.  Strict mode raises IndexError as
+    head_boundary_counts_batch does; CPU maps raise WcaError.
+    Device work: per width, one head-scoring and one top-k launch per weighting of its top-k configs (scores from the
+    capture's partials when it left them and w_coverage is not > 0, as _score_and_select chooses) and one aggregation
+    launch for all its (utterance, config) problems.  A top-k list for k is the last k entries of the list for the
+    largest k of the weighting (the ranking is ascending), so every k reads one ranking.  Configs that align the same
+    way (mean configs of one width whatever their weights, top-k configs whose capped k and weights agree) share one
+    problem.  Then one DTW launch for every problem of every width, one wca_boundary_hits launch, and the hits are the
+    only device->host copy."""
+    configs = [tuple(c) for c in configs]
+    B = len(tokens_list)
+    if len(ref_ends_list) != B or (ref_words_list is not None and len(ref_words_list) != B):
+        raise ValueError("tokens_list, ref_ends_list (and ref_words_list) must have the same batch length")
+    if not configs:
+        raise ValueError("alignment_config_counts_batch: no configuration given")
+    for width, aggr, topk, *_ in configs:
+        if aggr not in ("mean", "topk"):
+            raise ValueError(f"aggregation {aggr!r}: the sweep aligns with 'mean' or 'topk'")
+        if aggr == "topk" and not topk > 0:
+            raise AssertionError(f"topk={topk}: aggregation 'topk' needs topk > 0 (as force_align)")
+        if width not in maps_by_width:
+            raise ValueError(f"no maps for median-filter width {width}")
+    if B == 0:
+        return []
+    widths = list(dict.fromkeys(c[0] for c in configs))
+    maps = {}
+    for width in widths:
+        ms = list(maps_by_width[width])
+        if len(ms) != B:
+            raise ValueError(f"width {width}: {len(ms)} maps for {B} utterances")
+        for m in ms:
+            if not m.is_cuda:
+                raise _cabi.WcaError("alignment_config_counts: attention maps must be CUDA tensors (no CPU fallback exists)")
+        maps[width] = [m if m.is_contiguous() else m.contiguous() for m in ms]
+    shapes = np.array([m.shape for m in maps[widths[0]]], dtype=np.int64).reshape(B, 4)
+    L, H = int(shapes[0, 0]), int(shapes[0, 1])
+    for width in widths:
+        if not np.array_equal(np.array([m.shape for m in maps[width]], dtype=np.int64).reshape(B, 4), shapes):
+            raise ValueError("every width's maps must have the shapes of the first width's")
+    if (shapes[:, :2] != (L, H)).any():
+        raise ValueError("all utterances of a batch must have the same (layers, heads)")
+
+    # one problem per distinct alignment: (width, "mean") or (width, "topk", weights, k capped at L*H)
+    slot_of, slots = [], {}
+    for width, aggr, topk, wc, wr, wv in configs:
+        key = (width, "mean") if aggr == "mean" else (width, "topk", (wc, wr, wv), min(int(topk), L * H))
+        slot_of.append(slots.setdefault(key, len(slots)))
+    # problems slot-major, utterances within a slot; slots grouped by width
+    keys = sorted(slots, key=lambda k: (widths.index(k[0]), slots[k]))
+    renumber = {slots[k]: i for i, k in enumerate(keys)}
+    slot_of = np.array([renumber[s] for s in slot_of], dtype=np.int64)
+
+    sot_len = len(tokenizer.sot_sequence)
+    n_mean = (L - L // 2) * H  # "mean": layers L//2 .. L-1 (timing.py:87-88)
+    groups = []
+    for width in widths:
+        ms = maps[width]
+        dev = ms[0].device
+        wkeys = [k for k in keys if k[0] == width]
+        weightings = list(dict.fromkeys(k[2] for k in wkeys if k[1] == "topk"))
+        k_max = max([k[3] for k in wkeys if k[1] == "topk"], default=0)
+        parts, list_off = [], {}
+        if any(k[1] == "mean" for k in wkeys):
+            parts.append(torch.from_numpy(np.arange(L * H - n_mean, L * H, dtype=np.int32)).to(dev, non_blocking=True))
+            list_off["mean"] = 0
+        if weightings:
+            plan = _Plan(ms, sot_len, [k_max] * B)  # utterance b's ranking at b * k_max
+            for wt in weightings:
+                _, sel, _ = _score_and_select(plan, *wt)
+                list_off[wt] = sum(int(p.numel()) for p in parts)
+                parts.append(sel[: B * k_max])
+        sel = torch.cat(parts) if len(parts) > 1 else parts[0]
+        off = (np.array([m.data_ptr() for m in ms], dtype=np.int64) - ms[0].data_ptr()) // 4
+        utt, sel_off, n_sel = [], [], []
+        for k in wkeys:
+            utt.append(np.arange(B))
+            if k[1] == "mean":
+                sel_off.append(np.zeros(B, dtype=np.int64))  # every utterance reads the same list
+                n_sel.append(np.full(B, n_mean, dtype=np.int64))
+            else:
+                sel_off.append(list_off[k[2]] + np.arange(B) * k_max + (k_max - k[3]))
+                n_sel.append(np.full(B, k[3], dtype=np.int64))
+        utt = np.concatenate(utt)
+        groups.append((ms, sel, utt, off[utt], np.concatenate(sel_off), np.concatenate(n_sel)))
+    sh = _launch_problems(shapes[:, 2:], groups, tokens_list, tokenizer, aligned_unit_type)
+    return [c[slot_of] for c in _boundary_counts(sh, ref_ends_list, tolerance, ref_words_list)]
+
+
 def _boundary_counts(sh, ref_ends_list, tolerance, ref_words_list):
-    """The scoring half of head_boundary_counts_batch on the single-head alignments `sh` left on the device: per
-    utterance, an int64 (n_heads, 3) array of (hits, n_pred, n_ref).  One wca_boundary_hits launch, one copy back."""
+    """The scoring half of head_boundary_counts_batch on the alignments `sh` (_launch_problems) left on the device: per
+    utterance b, an int64 (n_b, 3) array of (hits, n_pred, n_ref), one row per problem of b in problem order.  One
+    wca_boundary_hits launch, one copy back."""
     B = len(sh.words_all)
     ref_ends = [np.asarray(r, dtype=np.float64).reshape(-1) for r in ref_ends_list]
     ref_ids = hyp_ids = None
@@ -633,19 +800,20 @@ def _boundary_counts(sh, ref_ends_list, tolerance, ref_words_list):
         # a reference shorter than its boundaries only gets here without predictions: its missing ids match nothing
         ref_ids = [np.pad(i, (0, len(e) - len(i)), constant_values=-1) for i, e in zip(ids[:B], ref_ends)]
         hyp_ids = ids[B:]
-    hits = torch.empty(max(int(sh.n_heads.sum()), 1), dtype=torch.int32, device=sh.times.device)
-    _cabi.boundary_hits(sh.times[1], sh.d_utts, np.repeat(np.arange(B), sh.n_heads), ref_ends, tolerance, hits,
+    hits = torch.empty(max(len(sh.utt_of), 1), dtype=torch.int32, device=sh.times.device)
+    _cabi.boundary_hits(sh.times[1], sh.d_utts, sh.utt_of, ref_ends, tolerance, hits,
                         ref_ids=ref_ids, hyp_ids=hyp_ids, n_pred=sh.recs["n_words"])
     hits_h = hits.cpu().numpy().astype(np.int64)  # the only device->host copy of the call
-    out, p = [], 0
+    order = np.argsort(sh.utt_of, kind="stable")  # problems by utterance, in problem order within one
+    bounds = np.concatenate([[0], np.cumsum(np.bincount(sh.utt_of, minlength=B))])
+    out = []
     for b in range(B):
-        k = int(sh.n_heads[b])
-        c = np.empty((k, 3), dtype=np.int64)
-        c[:, 0] = hits_h[p: p + k]
+        mine = order[bounds[b]: bounds[b + 1]]
+        c = np.empty((len(mine), 3), dtype=np.int64)
+        c[:, 0] = hits_h[mine]
         c[:, 1] = sh.n_words[b]
         c[:, 2] = len(ref_ends[b])
         out.append(c)
-        p += k
     return out
 
 
